@@ -9,12 +9,14 @@ a synthetic Zipf table of N_full = 1M haplotypes (alleles/locus 700/1200/600/250
 outputs, Plan B on.  One step = one pass of the hot path over the whole batch.
 
   python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--subjects S] [--haps H]
+                  [--dump-outputs DIR]
 
 value  : subjects/s, batch already resident in HBM, CUDA-event timed (max over ranks)
 e2e    : same through grimb_impute_host with pinned HOST buffers (H2D + kernel + D2H per step)
 roofline / cpu_baseline: see DESIGN.md "Measurement".  roofline.probe_bound places the dominant kernel against
 the random 32-byte-sector rate measured by tools/sector_peak.cu (the probe-bound roofline); e2e.link places the
 host-buffer leg against the time the PCIe link alone needs for the same bytes (tools/pcie_peak.py).
+--dump-outputs DIR: the results of the last timed `value` step (rank 0's batch) as DIR/*.npy, see dump_outputs().
 """
 import argparse
 import ctypes as C
@@ -327,6 +329,51 @@ def run_reference(args, rank):
     print(json.dumps(line))
 
 
+DUMP_MAX_SUBJECTS = 1 << 17     # ~29 MB of .npy files
+DUMP_SEED = 20261020
+
+
+def dump_outputs(out_dir, comp, words, pair_evals):
+    """Writes what one grimb_impute_device call returned for the batch, decoded per subject, so that two builds
+    can be compared file for file: word offsets come from an atomic cursor and differ from run to run, so the
+    files hold each subject's values, not the raw arrays.  Subjects: all of them, or a fixed seeded sample of
+    DUMP_MAX_SUBJECTS for larger batches (subject_index.npy).  Every subject of this workload is fully typed
+    with one population, i.e. a SIMPLE record (include/grimb200.h); any other kind is an error.
+      status [n], has_results [n], umug_prob [n] (the UMUG genotype's probability), pmug_rows [n],
+      pmug_phase [n][16] (phase id of PMUG row k in rank order, -1 past pmug_rows), pmug_prob [n][16] (0 past
+      pmug_rows), pair_evals [1]."""
+    from grim.imputation import _lib
+    S = len(comp)
+    idx = np.arange(S) if S <= DUMP_MAX_SUBJECTS else \
+        np.sort(np.random.RandomState(DUMP_SEED).choice(S, DUMP_MAX_SUBJECTS, replace=False))
+    c = comp[idx]
+    n = len(idx)
+    wf = words.view(np.float64)
+    rows = np.zeros(n, np.float32)
+    phase = np.full((n, 16), -1.0, np.float32)
+    prob = np.zeros((n, 16), np.float64)
+    for i in range(n):
+        kf, off = int(c["kind_flags"][i]), int(c["off"][i])
+        if (kf & 3) != _lib.KIND_SIMPLE:
+            raise RuntimeError("--dump-outputs: subject %d is not a SIMPLE record (kind_flags %#x)" % (idx[i], kf))
+        k = kf >> 4
+        if k == 15:        # long form: a count word, a word of phase ids, then the probabilities
+            k = min(16, int(words[off]))
+            ph, pr = int(words[off + 1]), wf[off + 2:off + 2 + k]
+        else:
+            ph, pr = int(c["phases"][i]), (wf[off:off + k] if kf & _lib.KIND_WORDS else c["total"][i])
+        rows[i] = k
+        phase[i, :k] = [(ph >> (4 * q)) & 15 for q in range(k)]
+        prob[i, :k] = pr
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {"subject_index": idx.astype(np.float64), "status": c["status"].astype(np.float32),
+              "has_results": ((c["kind_flags"] & _lib.KIND_HAS_RESULTS) != 0).astype(np.float32),
+              "umug_prob": c["total"].astype(np.float64), "pmug_rows": rows, "pmug_phase": phase, "pmug_prob": prob,
+              "pair_evals": np.array([pair_evals], np.float64)}
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 def workload_config(args):
     return {"workload": "C2: %d fully typed unambiguous 5-locus subjects, 1 population, synthetic Zipf table of %d "
                         "haplotypes, UMUG+PMUG top-10, Plan B on" % (args.subjects, args.haps),
@@ -356,7 +403,10 @@ def main():
     ap.add_argument("--c5-subjects", type=int, default=1 << 16)
     ap.add_argument("--c5m-haps", type=int, default=2000000, help="nine-locus table under a Plan_A_Matrix (0: skip)")
     ap.add_argument("--config-sample", type=int, default=300, help="subjects per configuration checked against the oracle")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the results of the last timed step as DIR/*.npy")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs applies to the GPU path")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local = int(os.environ.get("LOCAL_RANK", "0"))
@@ -547,6 +597,13 @@ def main():
     # `value`: back-to-back asynchronous calls (results and counters stay on the device until the end), so
     # the host turn-around between batches is hidden, as in a streaming caller
     ms_dev = timed(step_device_async, args.steps, args.warmup, drain=finish_device)
+    last_out = None
+    if args.dump_outputs and rank == 0:
+        # the engines alternate, so the last timed call wrote the buffers of engine (turn - 1) & 1; the untimed
+        # calls below reuse the first set
+        bufs, tot = (d_out, tot_dev) if ((turn[0] - 1) & 1) == 0 else (d_out2, tot_dev2)
+        last_out = (bufs["compact"].cpu().numpy().view(_lib.COMPACT_DTYPE),
+                    bufs["words"][:int(tot[0]) * 8].cpu().numpy().view(np.uint64), int(tot[4]))
     launches = (sum(lib.grimb_engine_launches(x) for x in engines) - launches0) * args.steps // (args.steps + args.warmup)
     for _ in range(max(5, min(20, args.steps))):   # per-kernel device times: synchronous calls, events inside the library
         step_device()
@@ -726,6 +783,8 @@ def main():
                                                      "note": "includes the host-side staging of bench.py's arrays"}
             except Exception as exc:   # the headline line must survive a failing sub-record
                 line["configs"] = {"error": repr(exc)}
+        if last_out is not None:
+            dump_outputs(args.dump_outputs, *last_out)
         print(json.dumps(line))
     if world > 1:
         dist.destroy_process_group()
