@@ -72,6 +72,11 @@ struct GrimbTables {
   TablesView view;
   int build_launches = 0;   // kernel launches of grimb_tables_build (0 for a table made from an image)
   float build_ms = 0.0f;    // device time of the build after the inputs were staged (CUDA events on the build's stream)
+#if GRIMB_KW == 1
+  char* fidx_mem = nullptr;   // FastIndex keys + fslot (derived from the image; tables the fast path serves only)
+  uint64_t fidx_bytes = 0;
+  FastIndex fidx = {nullptr, nullptr, 0};
+#endif
 };
 
 static void make_view(GrimbTables* t) {
@@ -132,6 +137,72 @@ __global__ void k_init_slots(HSlot* s, uint64_t n) {
 }
 
 static inline unsigned nblk(uint64_t n, unsigned t = 256) { return (unsigned)((n + t - 1) / t); }
+
+#if GRIMB_KW == 1
+// FastIndex insert: one thread per full haplotype (node ids [0, n_full): the full label comes first).
+// A key takes the first empty slot from its home sector on; one stored past its home sector sets the
+// home sector's flag.  Sectors never empty again, so every sector between a key's home and its slot is
+// full: a lookup may stop at the first sector with an empty slot.
+__global__ void k_fast_index(const hkey* __restrict__ node_key, const double* __restrict__ freq, uint32_t n,
+                             unsigned long long* keys, double* fslot, uint32_t sec_mask) {
+  const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= n) return;
+  const double f = freq[i];   // P == 1
+  if (!(f > 0)) return;       // the fast path treats f == 0 as absent
+  const unsigned long long key = node_key[i];
+  const uint32_t home = hash_key(key) & sec_mask;
+  for (uint32_t sec = home;; sec = (sec + 1) & sec_mask) {
+    unsigned long long* w = keys + 4ull * sec;
+    for (int j = 0; j < 4; ++j) {
+      // the first word of a sector may carry the flag: it is empty with the flag either way
+      unsigned long long flag = 0, old;
+      while ((old = atomicCAS(w + j, flag, flag | key)) != flag) {
+        if (j != 0 || (old & ~FIDX_FLAG) != 0) break;   // taken
+        flag = old;                                      // only the flag was set meanwhile
+      }
+      if (old == flag) {
+        fslot[4ull * sec + j] = f;
+        if (sec != home) atomicOr(keys + 4ull * home, FIDX_FLAG);
+        return;
+      }
+    }
+  }
+}
+
+// Builds t->fidx for a table the single-population fast path serves (L <= 5, P == 1); nothing otherwise.
+// GRIMB_FAST_INDEX_MULT (2..16) sets the slots per full haplotype.  Default 4: on B200 the 1M-haplotype table's
+// probe kernel takes the same time with 4 (32 MB of keys) as with 8 (64 MB), at half the memory.
+static cudaError_t build_fast_index(GrimbTables* t, int* launches) {
+  const ImageHeader& h = t->h;
+  if (h.L > 5 || h.P != 1) return cudaSuccess;
+  if (h.n_full > (1u << 30)) return cudaErrorInvalidValue;   // slot positions are 32-bit, load <= 1/2
+  uint64_t mult = 4;
+  if (const char* m = getenv("GRIMB_FAST_INDEX_MULT")) {
+    const long v = atol(m);
+    if (v >= 2 && v <= 16) mult = (uint64_t)v;
+  }
+  uint64_t n_slots = 4;
+  while (n_slots < mult * h.n_full && n_slots < (1ull << 31)) n_slots <<= 1;
+  cudaError_t e = cudaMalloc((void**)&t->fidx_mem, n_slots * 16);
+  if (e != cudaSuccess) {
+    t->fidx_mem = nullptr;
+    return e;
+  }
+  t->fidx_bytes = n_slots * 16;
+  unsigned long long* keys = (unsigned long long*)t->fidx_mem;
+  double* fslot = (double*)(t->fidx_mem + n_slots * 8);
+  t->fidx.keys = (const uint64_t*)keys;
+  t->fidx.fslot = fslot;
+  t->fidx.sec_mask = (uint32_t)(n_slots / 4 - 1);
+  e = cudaMemsetAsync(keys, 0, n_slots * 8, 0);
+  if (e != cudaSuccess) return e;
+  if (h.n_full) {
+    k_fast_index<<<nblk(h.n_full), 256>>>(t->view.node_key, t->view.freq, h.n_full, keys, fslot, t->fidx.sec_mask);
+    if (launches) ++*launches;
+  }
+  return cudaGetLastError();
+}
+#endif
 
 struct DevBuf {
   void* p = nullptr;
@@ -463,6 +534,9 @@ extern "C" int grimb_tables_build(const GrimbTableDesc* d, GrimbTables** out) {
     if (d_nconn) cudaFree(d_nconn);
     if (!ok) {
       if (t->image) cudaFree(t->image);
+#if GRIMB_KW == 1
+      if (t->fidx_mem) cudaFree(t->fidx_mem);
+#endif
       delete t;
     }
   };
@@ -796,6 +870,9 @@ extern "C" int grimb_tables_build(const GrimbTableDesc* d, GrimbTables** out) {
     }
   }
   CKT(cudaMemcpy(t->image, &h, sizeof(h), cudaMemcpyHostToDevice));
+#if GRIMB_KW == 1
+  CKT(build_fast_index(t, &launches));
+#endif
   cudaEventRecord(ev_b1, 0);
   CKT(cudaDeviceSynchronize());
   if (ev_b0 && ev_b1) cudaEventElapsedTime(&t->build_ms, ev_b0, ev_b1);
@@ -813,6 +890,9 @@ extern "C" int grimb_tables_free(GrimbTables* t) {
   if (!t) return GRIMB_OK;
   cudaSetDevice(t->device);
   cudaFree(t->image);
+#if GRIMB_KW == 1
+  cudaFree(t->fidx_mem);
+#endif
   delete t;
   return GRIMB_OK;
 }
@@ -830,6 +910,9 @@ extern "C" int grimb_tables_info(const GrimbTables* t, GrimbTableInfo* info) {
   info->n_conn_edges = (int64_t)t->h.n_conn_edges;
   info->n_slots = (int64_t)t->h.n_slots;
   info->device_bytes = (int64_t)t->h.bytes;
+#if GRIMB_KW == 1
+  info->device_bytes += (int64_t)t->fidx_bytes;
+#endif
   return GRIMB_OK;
 }
 
@@ -896,6 +979,17 @@ extern "C" int grimb_tables_from_image(const void* dev_image, int64_t bytes, int
     return fail(GRIMB_E_CUDA, cudaGetErrorString(e));
   }
   make_view(t);
+#if GRIMB_KW == 1
+  e = build_fast_index(t, nullptr);
+  if (e == cudaSuccess) e = cudaDeviceSynchronize();
+  if (e != cudaSuccess) {
+    cudaFree(t->fidx_mem);
+    cudaFree(t->image);
+    delete t;
+    return fail(e == cudaErrorMemoryAllocation ? GRIMB_E_NOMEM : GRIMB_E_CUDA,
+                std::string("fast-path index: ") + cudaGetErrorString(e));
+  }
+#endif
   *out = t;
   return GRIMB_OK;
 }
@@ -1131,6 +1225,53 @@ __device__ __forceinline__ void ht_lookup2(const HSlot* __restrict__ base, uint3
     else if (b1.node == GRIMB_NONE) {}
     else if (b1.key == k2) n2 = b1.node;
     else more2 = true;
+  }
+}
+
+// One 32-byte sector of the FastIndex (four keys) with one 256-bit load (sm_100: LDG.E.256).
+__device__ __forceinline__ void fidx_sector(const uint64_t* p, uint64_t (&w)[4]) {
+  uint32_t r0, r1, r2, r3, r4, r5, r6, r7;
+  asm volatile("ld.global.nc.v8.u32 {%0,%1,%2,%3,%4,%5,%6,%7}, [%8];"
+               : "=r"(r0), "=r"(r1), "=r"(r2), "=r"(r3), "=r"(r4), "=r"(r5), "=r"(r6), "=r"(r7)
+               : "l"(p));
+  w[0] = (uint64_t)r0 | ((uint64_t)r1 << 32);
+  w[1] = (uint64_t)r2 | ((uint64_t)r3 << 32);
+  w[2] = (uint64_t)r4 | ((uint64_t)r5 << 32);
+  w[3] = (uint64_t)r6 | ((uint64_t)r7 << 32);
+}
+
+// Examines sector `sec` of a probe for `key` (never 0): sets pos to the slot on a hit; returns true when
+// the next sector is needed -- no hit, no empty slot, and (home sector) the overflow flag set.
+__device__ __forceinline__ bool fidx_step(const uint64_t (&w)[4], uint64_t key, uint32_t sec, bool home, uint32_t& pos) {
+  const uint64_t w0 = w[0] & ~FIDX_FLAG;
+  if (w0 == key) pos = 4 * sec;
+  else if (w[1] == key) pos = 4 * sec + 1;
+  else if (w[2] == key) pos = 4 * sec + 2;
+  else if (w[3] == key) pos = 4 * sec + 3;
+  else return !(w0 == 0 || w[1] == 0 || w[2] == 0 || w[3] == 0) && (!home || (w[0] & FIDX_FLAG));
+  return false;
+}
+
+// Two independent FastIndex probes; the home sector of each is requested before either is examined (the
+// common case resolves both in that one round trip).  n1 / n2: slot positions, GRIMB_NONE when absent.
+__device__ __forceinline__ void fidx_lookup2(const FastIndex& X, uint64_t k1, bool p1, uint64_t k2, bool p2, uint32_t& n1,
+                                             uint32_t& n2) {
+  uint32_t h1 = hash_key(k1) & X.sec_mask, h2 = hash_key(k2) & X.sec_mask;
+  n1 = n2 = GRIMB_NONE;
+  uint64_t a[4] = {0, 0, 0, 0}, b[4] = {0, 0, 0, 0};
+  if (p1) fidx_sector(X.keys + 4ull * h1, a);
+  if (p2) fidx_sector(X.keys + 4ull * h2, b);
+  bool more1 = p1 && fidx_step(a, k1, h1, true, n1);
+  bool more2 = p2 && fidx_step(b, k2, h2, true, n2);
+  while (more1) {
+    h1 = (h1 + 1) & X.sec_mask;
+    fidx_sector(X.keys + 4ull * h1, a);
+    more1 = fidx_step(a, k1, h1, false, n1);
+  }
+  while (more2) {
+    h2 = (h2 + 1) & X.sec_mask;
+    fidx_sector(X.keys + 4ull * h2, b);
+    more2 = fidx_step(b, k2, h2, false, n2);
   }
 }
 
@@ -1395,37 +1536,37 @@ k_impute_fast(TablesView T, const GrimbConfig* __restrict__ cfg, GrimbBatch B, O
 
 
 // ------------------------------------------------------------------------------------------
-// Split form of the fast path: k_fast_probe (half-warp per subject: keys, probes, frequency loads)
-// hands the few phases whose two haplotypes are both in the table to k_fast_score (one LANE per
-// subject: epsilon schedule, sums, ranks, result record and rows).  The probe kernel carries no FP64
+// Split form of the fast path: k_fast_probe (half-warp per subject: keys, FastIndex probes) hands the
+// few phases whose two haplotypes are both in the table to k_fast_score (one LANE per subject: frequency
+// loads, epsilon schedule, sums, ranks, result record and rows).  The probe kernel carries no FP64
 // state, so it fits more warps per SM, and the scoring work -- which used 16 lanes per subject for
 // what is typically one or two candidate phases -- shrinks to a few instructions per subject.
-// Hand-over record: 96 bytes per subject in a device buffer owned by the engine.
+// Hand-over record: 48 bytes per subject in a device buffer owned by the engine.
 // ------------------------------------------------------------------------------------------
 constexpr int FAST_CMAX = 4;    // candidate phases k_fast_score keeps in registers (the usual subject has one or two)
 constexpr int FAST_CALL = 16;   // candidate phases a hand-over record holds (= every phase of a 5-locus subject)
 
-// Header and first candidate share one 32-byte sector: the usual subject (one candidate phase) costs one
-// sector written by the probe kernel and one read by the score kernel.  96 bytes = 3 sectors.  A subject with
-// more than FAST_CMAX candidate phases (rare) keeps them in a side record claimed from `extra`.
-// (round 2, later: the record is split -- a dense array of 32-byte heads, which is all the usual subject touches,
-// and a second array for candidates 2..4)
-struct __align__(32) FastHead {
-  uint32_t flags;        // bits 0-1 state (0 not for k_fast_score, 1 ready), 2-6 ncand, 7 both haplotypes equal
+// A candidate is the FastIndex slot positions (p1, p2) of its two haplotypes; k_fast_score reads their
+// frequencies from FastIndex.fslot.  The record is split: a dense array of 16-byte heads (flags and the
+// first candidate), which is all the usual subject (one candidate phase) touches, and a 32-byte record for
+// candidates 2..4.  A subject with more than FAST_CMAX candidate phases (rare) keeps them in a side
+// record claimed from `extra`.
+struct __align__(16) FastHead {
+  uint32_t flags;        // bits 0-1 state (0 not for k_fast_score, 1 ready), 2-6 ncand, 7 both haplotypes equal,
+                         // 16-31 candidate mask (bit i: phase i; candidates are stored in ascending phase order)
   uint32_t extra;        // ncand > FAST_CMAX: index of the subject's FastExtra
-  uint64_t phases;       // bit i: phase i is a candidate (candidates are stored in ascending phase order)
-  double f0[2];          // (f1, f2) of the first candidate phase
+  uint2 p0;              // (p1, p2) of the first candidate phase
 };
-struct __align__(64) FastMore {
-  double f[FAST_CMAX - 1][2];   // candidates 2..FAST_CMAX (ncand <= FAST_CMAX)
-  double pad[2];
+struct __align__(32) FastMore {
+  uint2 p[FAST_CMAX - 1];   // candidates 2..FAST_CMAX (ncand <= FAST_CMAX)
+  uint2 pad;
 };
 struct FastMid {
   FastHead* head;
   FastMore* more;
 };
 struct __align__(32) FastExtra {
-  double f[FAST_CALL][2];
+  uint2 p[FAST_CALL];
 };
 
 #ifndef FASTPROBE_MIN_BLOCKS
@@ -1465,7 +1606,7 @@ __device__ __forceinline__ void probe_load(ProbeIn& in, const GrimbBatch& B, uin
 
 template <bool PACKED>
 __global__ void __launch_bounds__(FAST_WARPS * 32, FASTPROBE_MIN_BLOCKS)
-k_fast_probe(TablesView T, GrimbBatch B, OutArrays O, FastMid mid, uint32_t* worklist,
+k_fast_probe(TablesView T, const FastIndex X, GrimbBatch B, OutArrays O, FastMid mid, uint32_t* worklist,
              unsigned int* worklist_n, FastExtra* __restrict__ extra, unsigned int* extra_n, uint32_t extra_cap, int nchain_ok,
              uint32_t s_begin) {
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
@@ -1479,8 +1620,6 @@ k_fast_probe(TablesView T, GrimbBatch B, OutArrays O, FastMid mid, uint32_t* wor
   uint64_t Mi = 0;
   for (int l = 0; l < L; ++l)
     if ((i >> l) & 1) Mi |= ((1ull << T.width[l]) - 1ull) << T.shift[l];
-  const uint32_t ht_mask = T.ht_mask[full];
-  const HSlot* __restrict__ ht_base = T.slots + T.ht_off[full];
   const uint32_t S = (uint32_t)B.n_subjects;               // subject indices fit 32 bits (worklists are uint32)
   const uint32_t stride = gridDim.x * FAST_WARPS * 2;
   uint32_t s = s_begin + (blockIdx.x * FAST_WARPS + warp) * 2 + half;   // subjects [s_begin, n_subjects)
@@ -1524,15 +1663,13 @@ k_fast_probe(TablesView T, GrimbBatch B, OutArrays O, FastMid mid, uint32_t* wor
       const bool last_het = (het >> (L - 1)) & 1u;
       const bool kept = i < nphase && !(ib & ~low) && (last_het || ib <= (low ^ ib));
       uint32_t n1, n2;
-      ht_lookup2(ht_base, ht_mask, key, kept && known1, key2, kept && known2, n1, n2);
-      const double f1 = n1 != GRIMB_NONE ? __ldg(T.freq + n1) : 0.0;   // P == 1
-      const double f2 = n2 != GRIMB_NONE ? __ldg(T.freq + n2) : 0.0;
-      const bool cand = kept && f1 > 0 && f2 > 0;
+      fidx_lookup2(X, key, kept && known1, key2, kept && known2, n1, n2);
+      const bool cand = kept && n1 != GRIMB_NONE && n2 != GRIMB_NONE;   // the index holds the haplotypes with f > 0
       const uint32_t cmask = (__ballot_sync(hmask, cand) >> hbase) & 0xFFFFu;
       ncand = __popc(cmask);
       state = 1;
       phases = cmask;   // the candidates' phase ids: k_fast_score reads them off the mask (q-th set bit)
-      double2* dst = nullptr;    // the side record of a long-form subject
+      uint2* dst = nullptr;      // the side record of a long-form subject
       if (ncand > FAST_CMAX) {   // rare: a side record (uniform in the half-warp)
         unsigned int x = 0;
         if (i == 0) x = atomicAdd(extra_n, 1u);
@@ -1542,16 +1679,14 @@ k_fast_probe(TablesView T, GrimbBatch B, OutArrays O, FastMid mid, uint32_t* wor
           state = 0;
           if (i == 0) worklist[atomicAdd(worklist_n, 1u)] = s;
         }
-        dst = reinterpret_cast<double2*>(&extra[x < extra_cap ? x : 0].f[0][0]);
+        dst = extra[x < extra_cap ? x : 0].p;
       }
       if (cand && state) {
         const uint32_t slot = __popc(cmask & ((1u << i) - 1u));
-        double2 v;
-        v.x = f1;
-        v.y = f2;
+        const uint2 v = make_uint2(n1, n2);
         if (dst) dst[slot] = v;
-        else if (slot == 0) *reinterpret_cast<double2*>(&mid.head[s].f0[0]) = v;
-        else *reinterpret_cast<double2*>(&mid.more[s].f[slot - 1][0]) = v;
+        else if (slot == 0) mid.head[s].p0 = v;
+        else mid.more[s].p[slot - 1] = v;
       }
     }
     if (!shape && typed != 0) {
@@ -1560,30 +1695,33 @@ k_fast_probe(TablesView T, GrimbBatch B, OutArrays O, FastMid mid, uint32_t* wor
     if (i == 0) {
       if (typed == 0)   // GRIMB_ST_SKIPPED: finished here
         O.r.compact[s] = make_compact(GRIMB_ST_SKIPPED, GRIMB_KIND_GENERAL, 0, 0xFFFFFFFFu, 0.0);
-      uint4 h1;   // header: state and candidate bookkeeping
-      h1.x = state | (ncand << 2) | (same << 7);
+      uint2 h1;   // header: state and candidate bookkeeping (p0 is written by the first candidate's lane)
+      h1.x = state | (ncand << 2) | (same << 7) | (phases << 16);
       h1.y = xslot;
-      h1.z = phases;
-      h1.w = 0;
-      reinterpret_cast<uint4*>(mid.head + s)[0] = h1;
+      *reinterpret_cast<uint2*>(mid.head + s) = h1;
     }
   }
 }
 
 // ---- more than FAST_CMAX candidate phases (rare): the WARP serves such a subject together, lane q = candidate q
-// (ascending phase), each lane reading its own (f1, f2) from the subject's side record once.  Same schedule as the
-// per-lane path below: first accepting round per candidate, minimum over the candidates, MaxProb / 100000, one more
-// evaluation, += in phase order, ranks by (probability desc, phase asc).
+// (ascending phase), each lane reading its own (p1, p2) from the subject's side record and their frequencies once.
+// Same schedule as the per-lane path below: first accepting round per candidate, minimum over the candidates,
+// MaxProb / 100000, one more evaluation, += in phase order, ranks by (probability desc, phase asc).
 struct LongCand {
   FastPair pr;
   double p;
   bool valid;
 };
 
-__device__ __forceinline__ void long_cand(LongCand& c, const FastExtra* ex, uint32_t q, uint32_t ncand, double m, bool same) {
+__device__ __forceinline__ void long_cand(LongCand& c, const FastExtra* ex, const double* __restrict__ fslot, uint32_t q,
+                                          uint32_t ncand, double m, bool same) {
   c.valid = q < ncand;
   double2 v = make_double2(0.0, 0.0);
-  if (c.valid) v = *reinterpret_cast<const double2*>(&ex->f[q][0]);
+  if (c.valid) {
+    const uint2 pp = ex->p[q];
+    v.x = __ldg(fslot + pp.x);
+    v.y = __ldg(fslot + pp.y);
+  }
   c.pr.f = v.x;
   c.pr.f2 = v.y;
   c.pr.same = same;
@@ -1610,11 +1748,11 @@ struct ScoreLong {
 };
 
 // called by all 32 lanes; every lane returns the same values
-__device__ __noinline__ void score_long_eval(const FastExtra* ex, uint32_t ncand, double m, bool same, const double* chain, int nchain,
-                                             ScoreLong& o) {
+__device__ __noinline__ void score_long_eval(const FastExtra* ex, const double* fslot, uint32_t ncand, double m, bool same,
+                                             const double* chain, int nchain, ScoreLong& o) {
   const int lane = threadIdx.x & 31;
   LongCand c;
-  long_cand(c, ex, (uint32_t)lane, ncand, m, same);
+  long_cand(c, ex, fslot, (uint32_t)lane, ncand, m, same);
   uint32_t rq = 99;
   if (c.pr.mpos) {
     int r = 0;
@@ -1656,11 +1794,11 @@ __device__ __noinline__ void score_long_eval(const FastExtra* ex, uint32_t ncand
 }
 
 // rows of the long form: words[0] = number of rows, words[1] = their phase ids (rank order), words[2 + k] = probability
-__device__ __noinline__ void score_long_rows(const FastExtra* ex, uint32_t ncand, double m, bool same, double e_fin, uint32_t cmask,
-                                             uint32_t np, uint64_t* words) {
+__device__ __noinline__ void score_long_rows(const FastExtra* ex, const double* fslot, uint32_t ncand, double m, bool same,
+                                             double e_fin, uint32_t cmask, uint32_t np, uint64_t* words) {
   const int lane = threadIdx.x & 31;
   LongCand c;
-  long_cand(c, ex, (uint32_t)lane, ncand, m, same);
+  long_cand(c, ex, fslot, (uint32_t)lane, ncand, m, same);
   const bool acc = c.pr.accept(e_fin);
   uint32_t am = __ballot_sync(0xFFFFFFFFu, acc);
   uint32_t rank = 0;   // by (probability desc, phase asc)
@@ -1689,7 +1827,7 @@ __device__ __noinline__ void score_long_rows(const FastExtra* ex, uint32_t ncand
 #define FASTSCORE_MIN_BLOCKS 8   /* 64 registers (a few spilled words): 0.046 ms per 2^20 subjects vs 0.048 at 6 CTAs, 0.052 unbounded (96) */
 #endif
 __global__ void __launch_bounds__(128, FASTSCORE_MIN_BLOCKS)
-k_fast_score(TablesView T, const GrimbConfig* __restrict__ cfg, GrimbBatch B, OutArrays O,
+k_fast_score(TablesView T, const FastIndex X, const GrimbConfig* __restrict__ cfg, GrimbBatch B, OutArrays O,
              const FastMid mid, const FastExtra* __restrict__ extra, uint32_t* worklist, unsigned int* worklist_n,
              uint32_t s_begin) {
   __shared__ double s_chain[FAST_MAX_ROUNDS];
@@ -1721,18 +1859,16 @@ k_fast_score(TablesView T, const GrimbConfig* __restrict__ cfg, GrimbBatch B, Ou
     double m = 0.0;
     uint32_t fl = 0, xslot = 0;
     uint32_t cmask = 0;    // candidate phases (bit i: phase i); candidate q is the q-th set bit
-    double2 f0 = make_double2(0.0, 0.0);
+    uint2 p0 = make_uint2(0u, 0u);
     if (s < S) {
-      // everything that does not depend on the header is requested with it: the prior (P == 1: one
-      // double per subject) and the first candidate's frequencies
-      const uint4* src = reinterpret_cast<const uint4*>(mid.head + s);
-      const uint4 h1 = src[0];
+      // the prior (P == 1: one double per subject) does not depend on the header: requested with it
+      const uint4 h1 = *reinterpret_cast<const uint4*>(mid.head + s);   // p0 is garbage unless ncand >= 1
       const uint32_t pi = batch_prior(B, s);
-      f0 = *reinterpret_cast<const double2*>(&mid.head[s].f0[0]);   // same sector as the header; garbage unless ncand >= 1
       m = __ldg(B.priors + pi);
       fl = h1.x;
       xslot = h1.y;
-      cmask = h1.z;
+      p0 = make_uint2(h1.z, h1.w);
+      cmask = fl >> 16;
       ready = (fl & 3u) == 1u;
     }
     const uint32_t ncand_all = ready ? ((fl >> 2) & 31u) : 0u;
@@ -1746,7 +1882,7 @@ k_fast_score(TablesView T, const GrimbConfig* __restrict__ cfg, GrimbBatch B, Ou
     for (uint32_t lm = __ballot_sync(0xFFFFFFFFu, long_form); lm; lm &= lm - 1) {
       const int o = __ffs(lm) - 1;
       ScoreLong r;
-      score_long_eval(extra + __shfl_sync(0xFFFFFFFFu, xslot, o), __shfl_sync(0xFFFFFFFFu, ncand_all, o), shfl_double(m, o),
+      score_long_eval(extra + __shfl_sync(0xFFFFFFFFu, xslot, o), X.fslot, __shfl_sync(0xFFFFFFFFu, ncand_all, o), shfl_double(m, o),
                       __shfl_sync(0xFFFFFFFFu, (int)same, o) != 0, s_chain, nchain, r);
       if (lane == o) sl = r;
     }
@@ -1754,13 +1890,26 @@ k_fast_score(TablesView T, const GrimbConfig* __restrict__ cfg, GrimbBatch B, Ou
     uint32_t rq[FAST_CMAX];
     bool acc[FAST_CMAX];
     uint32_t r_star = 99;
+    // the candidates' frequencies: every load is issued before any is used
+    uint2 pp[FAST_CMAX];
+    pp[0] = p0;
+#pragma unroll
+    for (int q = 1; q < FAST_CMAX; ++q) pp[q] = (uint32_t)q < ncand ? mid.more[s].p[q - 1] : make_uint2(0u, 0u);
 #pragma unroll
     for (int q = 0; q < FAST_CMAX; ++q) {
-      pf[q] = pf2[q] = prob[q] = 0.0;
+      pf[q] = pf2[q] = 0.0;
+      if ((uint32_t)q < ncand) {
+        pf[q] = __ldg(X.fslot + pp[q].x);
+        pf2[q] = __ldg(X.fslot + pp[q].y);
+      }
+    }
+#pragma unroll
+    for (int q = 0; q < FAST_CMAX; ++q) {
+      prob[q] = 0.0;
       rq[q] = 99;
       acc[q] = false;
       if ((uint32_t)q < ncand) {
-        const double2 v = q == 0 ? f0 : *reinterpret_cast<const double2*>(&mid.more[s].f[q - 1][0]);
+        const double2 v = make_double2(pf[q], pf2[q]);
         FastPair pr;
         pr.f = v.x;
         pr.f2 = v.y;
@@ -1772,8 +1921,6 @@ k_fast_score(TablesView T, const GrimbConfig* __restrict__ cfg, GrimbBatch B, Ou
         const bool tiny = !(b > 1.0e-280);
         pr.lo = tiny ? -1.0 : b * (1.0 - 0x1p-50);
         pr.hi = tiny ? __longlong_as_double(0x7ff0000000000000LL) : b * (1.0 + 0x1p-50);
-        pf[q] = v.x;
-        pf2[q] = v.y;
         double p = v.x * v.y * m;
         if (!same) p = p * 2;
         prob[q] = p;
@@ -1866,7 +2013,7 @@ k_fast_score(TablesView T, const GrimbConfig* __restrict__ cfg, GrimbBatch B, Ou
       const uint32_t ph = __shfl_sync(0xFFFFFFFFu, cmask, o);
       const uint64_t at = (uint64_t)__shfl_sync(0xFFFFFFFFu, (uint32_t)my, o) |
                           ((uint64_t)__shfl_sync(0xFFFFFFFFu, (uint32_t)(my >> 32), o) << 32);
-      score_long_rows(extra + __shfl_sync(0xFFFFFFFFu, xslot, o), __shfl_sync(0xFFFFFFFFu, ncand_all, o), shfl_double(m, o),
+      score_long_rows(extra + __shfl_sync(0xFFFFFFFFu, xslot, o), X.fslot, __shfl_sync(0xFFFFFFFFu, ncand_all, o), shfl_double(m, o),
                       __shfl_sync(0xFFFFFFFFu, (int)same, o) != 0, shfl_double(sl.e_fin, o), ph, __shfl_sync(0xFFFFFFFFu, np, o),
                       R.words + at);
     }
@@ -2674,6 +2821,8 @@ static int launch_warp(GrimbEngine* e, const GrimbConfig* cfg, const GrimbBatch*
   if (tv.L <= 5 && tv.P == 1) {
     const uint64_t groups = ((uint64_t)n + FAST_WARPS * 2 - 1) / (FAST_WARPS * 2);
     if (e->fast_split) {
+      const FastIndex& fidx = e->tables->fidx;
+      if (!fidx.keys) return fail(GRIMB_E_ARG, "table has no fast-path index");
       CK(e->mid.reserve((size_t)batch->n_subjects * (sizeof(FastHead) + sizeof(FastMore)) + 256));
       FastMid midv;
       midv.head = (FastHead*)e->mid.p;
@@ -2692,17 +2841,17 @@ static int launch_warp(GrimbEngine* e, const GrimbConfig* cfg, const GrimbBatch*
       unsigned int* ovf_n = (unsigned int*)(e->d_counters + CNT_OVERFLOW);
       if (tm) CK(cudaEventRecord(e->ev[0], st));
       if (batch->packed_keys)
-        k_fast_probe<true><<<(unsigned)fgp, FAST_WARPS * 32, 0, st>>>(tv, rb, O, midv, (uint32_t*)e->worklist.p, cnt,
+        k_fast_probe<true><<<(unsigned)fgp, FAST_WARPS * 32, 0, st>>>(tv, fidx, rb, O, midv, (uint32_t*)e->worklist.p, cnt,
                                                                     (FastExtra*)e->overflow.p, ovf_n, extra_cap, eps > 0 ? 0 : 1, (uint32_t)s_begin);
       else
-        k_fast_probe<false><<<(unsigned)fgp, FAST_WARPS * 32, 0, st>>>(tv, rb, O, midv, (uint32_t*)e->worklist.p, cnt,
+        k_fast_probe<false><<<(unsigned)fgp, FAST_WARPS * 32, 0, st>>>(tv, fidx, rb, O, midv, (uint32_t*)e->worklist.p, cnt,
                                                                      (FastExtra*)e->overflow.p, ovf_n, extra_cap, eps > 0 ? 0 : 1, (uint32_t)s_begin);
       CK(cudaGetLastError());
       if (tm) CK(cudaEventRecord(e->ev[1], st));
       uint64_t sg = ((uint64_t)n + 127) / 128;
       if (sg > (uint64_t)e->sm_count * 16) sg = (uint64_t)e->sm_count * 16;
       if (tm) CK(cudaEventRecord(e->ev_score[0], st));
-      k_fast_score<<<(unsigned)sg, 128, 0, st>>>(tv, e->d_cfg, rb, O, midv, (const FastExtra*)e->overflow.p,
+      k_fast_score<<<(unsigned)sg, 128, 0, st>>>(tv, fidx, e->d_cfg, rb, O, midv, (const FastExtra*)e->overflow.p,
                                                 (uint32_t*)e->worklist.p, cnt, (uint32_t)s_begin);
       CK(cudaGetLastError());
       if (tm) CK(cudaEventRecord(e->ev_score[1], st));

@@ -1,8 +1,9 @@
 // grimb_tables.h -- device view of the frequency store and the probe primitives.
 //
 // Layout in HBM (DESIGN.md "Data layout"):
-//   slots      open-addressing hash table, one region per locus-subset label (so the
-//              full-label region of a 1M-haplotype table is 32 MB and stays L2-resident);
+//   slots      open-addressing hash table, one region per locus-subset label (the full-label
+//              region of a 1M-haplotype table is 128 MB at load 1/8, larger than the L2; the
+//              single-population fast path probes the FastIndex below instead);
 //              16-byte slots {packed key, node id}, load factor <= 0.5, linear probing, one
 //              128-bit load per probe (two slots per 32-byte sector); 32-byte slots when the
 //              packed key is 128 bits wide (GRIMB_KW = 2).
@@ -53,6 +54,24 @@ struct TablesView {
   const uint32_t* cn_cnt;
   const uint32_t* cn_adj;
 };
+
+#if GRIMB_KW == 1
+// Key-only index of the full haplotypes with freq > 0, for the single-population fast path
+// (k_fast_probe / k_fast_score; L <= 5, P == 1).  Derived from the image on every device that holds
+// one (grimb_tables_build, grimb_tables_from_image), never stored in it.
+//   keys   [sec_mask + 1][4] packed keys, four to a 32-byte sector, 0 = empty (every field of a full
+//          key is >= 1).  Home sector hash_key(key) & sec_mask, linear probing by sector.  Bit 63 of a
+//          sector's first word (keys have <= 63 bits) is set when a key whose home is this sector is
+//          stored further on: a miss reads one sector unless it is set.  At 4 slots per haplotype the
+//          1M-haplotype table's keys are 32 MB, inside the L2.
+//   fslot  frequency of the key in the same slot (k_fast_score reads it; the probe kernel never does)
+struct FastIndex {
+  const uint64_t* keys;
+  const double* fslot;
+  uint32_t sec_mask;
+};
+#define FIDX_FLAG (1ull << 63)
+#endif
 
 GD uint64_t key_field(const TablesView& T, hkey key, int locus) {
   return (uint64_t)(key >> T.shift[locus]) & ((1ull << T.width[locus]) - 1ull);
