@@ -304,7 +304,9 @@ int64_t grimb_engine_launches(const GrimbEngine* e);
  * single-population probe kernel (k_fast_probe; k_impute_fast when GRIMB_FAST_SPLIT=0), 1 k_impute,
  * 2 k_impute_typed, 4 k_fast_score; negative if that kernel was not launched.  which = 3
  * (diagnostic): number of subjects the warp-per-subject kernels of the last call handed on to
- * k_impute. */
+ * k_impute.  which = 6 (diagnostic): the probe kernel of the engine's last split fast-path launch,
+ * 2 the two-level k_fast_probe2 (packed batch), 1 k_fast_probe on a packed batch, 0 k_fast_probe on
+ * the general batch form, -1 none yet. */
 double grimb_engine_kernel_ms(const GrimbEngine* e, int which);
 
 /* ------------------------------------------------------------------------------------------

@@ -1703,6 +1703,252 @@ k_fast_probe(TablesView T, const FastIndex X, GrimbBatch B, OutArrays O, FastMid
   }
 }
 
+// ---- two-level form of k_fast_probe (packed batches; the default, GRIMB_FAST_PROBE=1 selects the kernel above).
+// A phase is a candidate only when BOTH of its haplotypes are in the table, and the usual first haplotype is not
+// (DESIGN §4: 1.5 of ~14 eligible phases per subject hit).  Level 1 probes the first haplotype of every eligible
+// phase; each hit appends (second key, p1, subject, phase) to a per-warp queue in shared memory, and the queue is
+// drained 32 entries at a time, one second probe per lane, with its loads in flight together with the next
+// iteration's level-1 loads.  The hand-over record is the one k_fast_probe writes, bit for bit.
+// Warp-uniform by construction: the loop runs while the warp's first subject is < S, every lane takes every
+// branch that holds a __shfl / __ballot / __match_any / __syncwarp, and lanes of subjects >= S only mask.
+#ifndef FASTPROBE2_MIN_BLOCKS
+#define FASTPROBE2_MIN_BLOCKS 4   /* 63 registers, 0 spills, 32 warps/SM: 0.146 ms vs 0.196 at 5 CTAs (48 registers,
+                                     130 B spilled), 0.282 at 6 (40 registers, 238 B spilled) */
+#endif
+constexpr uint32_t PQ_CAP = 128;   // queue entries per warp (a power of two; the bound is argued at the drain)
+constexpr uint32_t PQ_DRAIN = 32;  // a drain serves at most one entry per lane
+constexpr uint32_t PQ_HIGH = 64;   // after an iteration's enqueue the warp drains (without overlap) while >= this
+
+struct ProbeQueue {
+  uint64_t key[PQ_CAP];   // the second haplotype of the phase
+  uint32_t p1[PQ_CAP];    // FastIndex slot of the first haplotype
+  uint32_t s[PQ_CAP];     // subject
+  uint8_t ph[PQ_CAP];     // phase
+};
+
+// one queue entry per lane, its second probe's home sector requested (what the entry holds besides the key is
+// read again from the queue when the sector has arrived)
+struct Drain {
+  uint64_t key, w[4];
+  uint32_t sec;
+  bool v;
+};
+
+// Entries [qh, qh + min(qn, 32)) of the ring, less the entries of the subject that continues past the window:
+// entries of one subject are contiguous and at most 16, so a drain of a queue holding more than 32 entries
+// takes at least 17 and only whole subjects.  Reads stay within the qn <= 110 live entries (see the loop).
+__device__ __forceinline__ void drain_issue(const ProbeQueue& q, const FastIndex& X, uint32_t qh, uint32_t qn, int lane,
+                                            Drain& d) {
+  const uint32_t e = (qh + (uint32_t)lane) & (PQ_CAP - 1u);
+  d.v = (uint32_t)lane < qn;   // lane < 32
+  if (qn > PQ_DRAIN && q.s[e] == q.s[(qh + PQ_DRAIN) & (PQ_CAP - 1u)]) d.v = false;   // entry 32 is live when qn > 32
+  d.key = q.key[e];
+  d.sec = hash_key(d.key) & X.sec_mask;
+  d.w[0] = d.w[1] = d.w[2] = d.w[3] = 0;
+  if (d.v) fidx_sector(X.keys + 4ull * d.sec, d.w);
+}
+
+// The second probes of a drain resolved; each subject of the window gets its hand-over record (same layout and
+// values as k_fast_probe).  Returns the entries consumed.  Called by all 32 lanes.
+__device__ __forceinline__ uint32_t drain_finish(const ProbeQueue& q, Drain& d, const FastIndex& X, uint32_t qh, FastMid mid,
+                                                 uint32_t* worklist, unsigned int* worklist_n, FastExtra* __restrict__ extra,
+                                                 unsigned int* extra_n, uint32_t extra_cap, int lane) {
+  const uint32_t FULL = 0xFFFFFFFFu;
+  uint32_t p2 = GRIMB_NONE;
+  bool more = d.v && fidx_step(d.w, d.key, d.sec, true, p2);
+  while (more) {   // continuation sectors (rare; per lane, no warp collective inside)
+    d.sec = (d.sec + 1) & X.sec_mask;
+    fidx_sector(X.keys + 4ull * d.sec, d.w);
+    more = fidx_step(d.w, d.key, d.sec, false, p2);
+  }
+  const uint32_t e = (qh + (uint32_t)lane) & (PQ_CAP - 1u);
+  // subject indices are < S <= 2^32 - 1: the invalid lanes' marker never equals a valid lane's subject
+  const uint32_t s = d.v ? q.s[e] : 0xFFFFFFFFu;
+  const bool cand = d.v && p2 != GRIMB_NONE;
+  const uint32_t taken = __ballot_sync(FULL, d.v);
+  const uint32_t grp = __match_any_sync(FULL, s);   // the lanes of my subject: contiguous (invalid lanes: the tail)
+  const uint32_t cb = __ballot_sync(FULL, cand) & grp;
+  const int leader = __ffs(grp) - 1;
+  const uint32_t ncand = __popc(cb);
+  // phase mask of the subject's candidates: segmented OR over the group (contiguous, <= 16 lanes)
+  uint32_t cm = cand ? (1u << q.ph[e]) : 0u;
+#pragma unroll
+  for (int k = 1; k < 16; k <<= 1) {
+    const uint32_t t = __shfl_down_sync(FULL, cm, k);
+    if (((grp >> lane) >> k) & 1u) cm |= t;   // lane + k is in my group (0 past lane 31)
+  }
+  const bool lead = d.v && lane == leader;
+  const bool longf = ncand > (uint32_t)FAST_CMAX;   // uniform in the group
+  unsigned int x = 0;
+  if (lead && longf) x = atomicAdd(extra_n, 1u);
+  x = __shfl_sync(FULL, x, leader);
+  const bool ok = !longf || x < extra_cap;   // no side record left: the general kernel serves the subject
+  if (cand && ok) {
+    const uint32_t slot = __popc(cb & ((1u << lane) - 1u));
+    const uint2 v = make_uint2(q.p1[e], p2);
+    if (longf) extra[x].p[slot] = v;
+    else if (slot == 0) mid.head[s].p0 = v;
+    else mid.more[s].p[slot - 1] = v;
+  }
+  if (lead) {
+    if (!ok) worklist[atomicAdd(worklist_n, 1u)] = s;
+    uint2 h1;
+    h1.x = (ok ? 1u : 0u) | (ncand << 2) | (cm << 16);   // same = 0: homozygous subjects never enter the queue
+    h1.y = longf ? x : 0u;
+    *reinterpret_cast<uint2*>(mid.head + s) = h1;
+  }
+  return __popc(taken);
+}
+
+__global__ void __launch_bounds__(FAST_WARPS * 32, FASTPROBE2_MIN_BLOCKS)
+k_fast_probe2(TablesView T, const FastIndex X, GrimbBatch B, OutArrays O, FastMid mid, uint32_t* worklist,
+              unsigned int* worklist_n, FastExtra* __restrict__ extra, unsigned int* extra_n, uint32_t extra_cap,
+              int nchain_ok, uint32_t s_begin) {
+  __shared__ ProbeQueue s_q[FAST_WARPS];
+  const uint32_t FULL = 0xFFFFFFFFu;
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+  const int half = lane >> 4, i = lane & 15;
+  ProbeQueue& q = s_q[warp];
+  const int L = T.L;
+  const int nphase = 1 << (L - 1);
+  uint64_t Mi = 0;
+  for (int l = 0; l < L; ++l)
+    if ((i >> l) & 1) Mi |= ((1ull << T.width[l]) - 1ull) << T.shift[l];
+  const uint32_t ib = (uint32_t)i;
+  const uint32_t lt = (1u << lane) - 1u;
+  const uint32_t S = (uint32_t)B.n_subjects;   // subject indices fit 32 bits (worklists are uint32)
+  const uint32_t stride = gridDim.x * FAST_WARPS * 4;
+  // the warp serves subjects s0 .. s0+3 per iteration: lane (half h, phase i) owns phase i of s0+h and s0+2+h.
+  // s0 < S in the loop, so "s0 + k < S" is written S - s0 > k (no 32-bit overflow)
+  uint32_t s0 = s_begin + (blockIdx.x * FAST_WARPS + warp) * 4;
+  uint32_t qh = 0, qn = 0;   // ring head and fill (warp-uniform)
+  uint4 nk[2];
+  uint32_t nf[2];
+#pragma unroll
+  for (int u = 0; u < 2; ++u) {
+    nk[u] = make_uint4(0u, 0u, 0u, 0u);
+    nf[u] = 0x8000u;
+    if (s0 < S && S - s0 > (uint32_t)(2 * u + half)) {
+      nk[u] = __ldg(reinterpret_cast<const uint4*>(B.packed_keys) + s0 + 2 * u + half);
+      nf[u] = B.packed_flags[s0 + 2 * u + half];
+    }
+  }
+  Drain d;
+  while (s0 < S) {
+    // level 1: phase i's first haplotype, for both subjects of the lane; both sectors requested before either is examined
+    uint64_t key[2], key2[2], w[2][4];
+    uint32_t sec[2], cf[2];
+    bool pr[2];
+#pragma unroll
+    for (int u = 0; u < 2; ++u) {
+      const uint32_t fl = cf[u] = nf[u];
+      const bool shape = S - s0 > (uint32_t)(2 * u + half) && !(fl & 0x8000u) && nchain_ok;   // packed: not skipped = shape
+      const uint64_t k0 = (uint64_t)nk[u].x | ((uint64_t)nk[u].y << 32), k1 = (uint64_t)nk[u].z | ((uint64_t)nk[u].w << 32);
+      const uint32_t het = fl & 31u, unk0 = (fl >> 5) & 31u, unk1 = (fl >> 10) & 31u;
+      const uint64_t D = k0 ^ k1;
+      key[u] = k0 ^ (D & Mi);
+      key2[u] = key[u] ^ D;
+      const bool known1 = ((unk0 & ~ib) | (unk1 & ib)) == 0, known2 = ((unk1 & ~ib) | (unk0 & ib)) == 0;
+      const uint32_t low = het & ((uint32_t)nphase - 1u);
+      const bool last_het = (het >> (L - 1)) & 1u;
+      const bool kept = i < nphase && !(ib & ~low) && (last_het || ib <= (low ^ ib));
+      // a phase with an unknown allele on either side cannot be a candidate: not probed at all
+      pr[u] = shape && kept && known1 && known2;
+      sec[u] = hash_key(key[u]) & X.sec_mask;
+      w[u][0] = w[u][1] = w[u][2] = w[u][3] = 0;
+      if (pr[u]) fidx_sector(X.keys + 4ull * sec[u], w[u]);
+    }
+    // level 2, overlapped: a queue holding 32 or more entries is drained with this iteration's level-1 loads in flight
+    const bool drain_now = qn >= PQ_DRAIN;
+    if (drain_now) drain_issue(q, X, qh, qn, lane, d);
+    uint32_t p1[2];
+#pragma unroll
+    for (int u = 0; u < 2; ++u) {
+      p1[u] = GRIMB_NONE;
+      bool more = pr[u] && fidx_step(w[u], key[u], sec[u], true, p1[u]);
+      while (more) {
+        sec[u] = (sec[u] + 1) & X.sec_mask;
+        fidx_sector(X.keys + 4ull * sec[u], w[u]);
+        more = fidx_step(w[u], key[u], sec[u], false, p1[u]);
+      }
+    }
+    // the next iteration's inputs, requested once the level-1 sectors are consumed (fewer registers at the peak)
+    const bool last = stride >= S - s0;
+#pragma unroll
+    for (int u = 0; u < 2; ++u) {
+      nf[u] = 0x8000u;
+      if (!last && S - s0 - stride > (uint32_t)(2 * u + half)) {
+        nk[u] = __ldg(reinterpret_cast<const uint4*>(B.packed_keys) + s0 + stride + 2 * u + half);
+        nf[u] = B.packed_flags[s0 + stride + 2 * u + half];
+      }
+    }
+    if (drain_now) {
+      const uint32_t n = drain_finish(q, d, X, qh, mid, worklist, worklist_n, extra, extra_n, extra_cap, lane);
+      qh += n;
+      qn -= n;
+      __syncwarp();   // the drained entries were read before this iteration's enqueue may reuse their slots
+    }
+    // level-1 results.  Homozygous subjects (both haplotypes one key) are decided here, as are subjects without a
+    // level-1 hit; the others enqueue one entry per hit phase, subject by subject (ballot order: s0, s0+1, s0+2, s0+3)
+    uint32_t base = qh + qn;
+#pragma unroll
+    for (int u = 0; u < 2; ++u) {
+      const uint32_t s = s0 + 2 * u + half;
+      const uint32_t fl = cf[u];
+      const bool inb = S - s0 > (uint32_t)(2 * u + half);
+      const bool shape = inb && !(fl & 0x8000u) && nchain_ok;
+      const bool same = (fl & 31u) == 0u;
+      const bool hit = p1[u] != GRIMB_NONE;   // pr[u] implied
+      const uint32_t enq = __ballot_sync(FULL, hit && !same);
+      const uint32_t hh = (enq >> (half << 4)) & 0xFFFFu;   // the level-1 hits of a heterozygous subject
+      if (hit && !same) {
+        // bound: qn <= 46 after the drain above (see below), plus at most 64 entries this iteration: <= 110 < PQ_CAP
+        const uint32_t e = (base + __popc(enq & lt)) & (PQ_CAP - 1u);
+        q.key[e] = key2[u];
+        q.p1[e] = p1[u];
+        q.s[e] = s;
+        q.ph[e] = (uint8_t)i;
+      }
+      base += __popc(enq);
+      if (i == 0 && inb) {
+        if (!shape) {
+          if (fl & 0x8000u)   // GRIMB_ST_SKIPPED: finished here
+            O.r.compact[s] = make_compact(GRIMB_ST_SKIPPED, GRIMB_KIND_GENERAL, 0, 0xFFFFFFFFu, 0.0);
+          else
+            worklist[atomicAdd(worklist_n, 1u)] = s;
+          mid.head[s] = FastHead{0u, 0u, make_uint2(0u, 0u)};
+        } else if (same) {   // phase 0 only; its second haplotype is its first
+          mid.head[s] = FastHead{1u | (hit ? (1u << 2) | (1u << 16) : 0u) | (1u << 7), 0u, make_uint2(p1[u], p1[u])};
+        } else if (hh == 0u) {
+          mid.head[s] = FastHead{1u, 0u, make_uint2(0u, 0u)};
+        }
+      }
+    }
+    qn = base - qh;
+    __syncwarp();   // the enqueued entries are visible to every lane of the next drain
+    // bound: qn <= 110 here.  Each drain of more than 32 entries takes at least 17, so this leaves qn <= 63, the
+    // overlapped drain of the next iteration leaves qn <= 46 (or <= 31 when it does not run) and the next
+    // enqueue adds <= 64.  Adversarial batches only: on the benchmark's batch the queue peaks at 56 entries and
+    // this loop never runs (tools/probe_queue_sim.py)
+    while (qn >= PQ_HIGH) {
+      drain_issue(q, X, qh, qn, lane, d);
+      const uint32_t n = drain_finish(q, d, X, qh, mid, worklist, worklist_n, extra, extra_n, extra_cap, lane);
+      qh += n;
+      qn -= n;
+      __syncwarp();
+    }
+    if (last) break;
+    s0 += stride;
+  }
+  while (qn > 0) {   // flush: every entry left belongs to a whole subject
+    drain_issue(q, X, qh, qn, lane, d);
+    const uint32_t n = drain_finish(q, d, X, qh, mid, worklist, worklist_n, extra, extra_n, extra_cap, lane);
+    qh += n;
+    qn -= n;
+    __syncwarp();
+  }
+}
+
 // ---- more than FAST_CMAX candidate phases (rare): the WARP serves such a subject together, lane q = candidate q
 // (ascending phase), each lane reading its own (p1, p2) from the subject's side record and their frequencies once.
 // Same schedule as the per-lane path below: first accepting round per candidate, minimum over the candidates,
@@ -2559,6 +2805,8 @@ struct GrimbEngine {
   int sm_count = 0;
   int fast_path = 1; // GRIMB_FAST=0 disables the warp-per-subject kernel (debugging / A-B runs)
   int fast_split = 1; // k_fast_probe + k_fast_score (default); GRIMB_FAST_SPLIT=0: the fused k_impute_fast
+  int fast_probe = 2; // packed batches: k_fast_probe2 (default); GRIMB_FAST_PROBE=1: the one-level k_fast_probe
+  int last_probe = -1; // last split fast-path launch: 2 k_fast_probe2, 1 k_fast_probe (packed), 0 k_fast_probe (general form)
   int timing = 1;     // CUDA events around the kernels in the device-pointer form (GRIMB_KERNEL_EVENTS=0: none)
   int timing_host = 0;   // ... in the chunked host-pointer form (GRIMB_HOST_EVENTS=1)
   DevBuf mid;         // hand-over records of the split fast path
@@ -2661,6 +2909,8 @@ extern "C" int grimb_engine_create(const GrimbTables* t, int64_t workspace_bytes
   if (fp && fp[0] == '0') e->fast_path = 0;
   const char* fsp = getenv("GRIMB_FAST_SPLIT");
   if (fsp && fsp[0] == '0') e->fast_split = 0;
+  const char* fpr = getenv("GRIMB_FAST_PROBE");
+  if (fpr && fpr[0] == '1') e->fast_probe = 1;
   const char* kev = getenv("GRIMB_KERNEL_EVENTS");
   if (kev && kev[0] == '0') e->timing = 0;
   const char* hev = getenv("GRIMB_HOST_EVENTS");
@@ -2728,6 +2978,7 @@ extern "C" int64_t grimb_engine_launches(const GrimbEngine* e) { return e ? e->l
 // has finished.  < 0 if not launched.  which = 3: subjects the last call handed on to k_impute.
 extern "C" double grimb_engine_kernel_ms(const GrimbEngine* e, int which) {
   if (e && which == 3) return e->last_worklist;
+  if (e && which == 6) return (double)e->last_probe;
   if (e && which == 5) {   // k_impute_slots
     float ms5 = -1.f;
     if (!e->ev_slots_valid || cudaEventElapsedTime(&ms5, e->ev_slots[0], e->ev_slots[1]) != cudaSuccess) {
@@ -2840,12 +3091,23 @@ static int launch_warp(GrimbEngine* e, const GrimbConfig* cfg, const GrimbBatch*
       CK(e->overflow.reserve((size_t)extra_cap * sizeof(FastExtra) + 64));
       unsigned int* ovf_n = (unsigned int*)(e->d_counters + CNT_OVERFLOW);
       if (tm) CK(cudaEventRecord(e->ev[0], st));
-      if (batch->packed_keys)
+      if (batch->packed_keys && e->fast_probe == 2) {
+        uint64_t g2 = (uint64_t)e->sm_count * FASTPROBE2_MIN_BLOCKS;
+        const uint64_t quads = ((uint64_t)n + FAST_WARPS * 4 - 1) / (FAST_WARPS * 4);
+        if (g2 > quads) g2 = quads;
+        k_fast_probe2<<<(unsigned)g2, FAST_WARPS * 32, 0, st>>>(tv, fidx, rb, O, midv, (uint32_t*)e->worklist.p, cnt,
+                                                             (FastExtra*)e->overflow.p, ovf_n, extra_cap, eps > 0 ? 0 : 1,
+                                                             (uint32_t)s_begin);
+        e->last_probe = 2;
+      } else if (batch->packed_keys) {
         k_fast_probe<true><<<(unsigned)fgp, FAST_WARPS * 32, 0, st>>>(tv, fidx, rb, O, midv, (uint32_t*)e->worklist.p, cnt,
                                                                     (FastExtra*)e->overflow.p, ovf_n, extra_cap, eps > 0 ? 0 : 1, (uint32_t)s_begin);
-      else
+        e->last_probe = 1;
+      } else {
         k_fast_probe<false><<<(unsigned)fgp, FAST_WARPS * 32, 0, st>>>(tv, fidx, rb, O, midv, (uint32_t*)e->worklist.p, cnt,
                                                                      (FastExtra*)e->overflow.p, ovf_n, extra_cap, eps > 0 ? 0 : 1, (uint32_t)s_begin);
+        e->last_probe = 0;
+      }
       CK(cudaGetLastError());
       if (tm) CK(cudaEventRecord(e->ev[1], st));
       uint64_t sg = ((uint64_t)n + 127) / 128;
