@@ -86,7 +86,7 @@ int grimb_abi_version(void);
 const char* grimb_last_error(void);
 /* sizeof of an ABI struct as the library was compiled, for bindings to check their mirror of it: 0 GrimbConfig,
  * 1 GrimbTableDesc, 2 GrimbTextDesc, 3 GrimbBatch, 4 GrimbResults, 5 GrimbTextOut, 6 GrimbFileStats,
- * 7 GrimbTableInfo; -1 otherwise. */
+ * 7 GrimbTableInfo, 8 GrimbRows; -1 otherwise. */
 int64_t grimb_struct_size(int32_t which);
 
 int grimb_tables_build(const GrimbTableDesc* desc, GrimbTables** out);
@@ -306,8 +306,69 @@ int64_t grimb_engine_launches(const GrimbEngine* e);
  * (diagnostic): number of subjects the warp-per-subject kernels of the last call handed on to
  * k_impute.  which = 6 (diagnostic): the probe kernel of the engine's last split fast-path launch,
  * 2 the two-level k_fast_probe2 (packed batch), 1 k_fast_probe on a packed batch, 0 k_fast_probe on
- * the general batch form, -1 none yet. */
+ * the general batch form, -1 none yet.  which = 7: the last grimb_batch_from_genotypes (k_geno_encode, plus the
+ * allele-offset scan and k_geno_fill when it built the general form); which = 8: the last grimb_results_rows
+ * (k_rows_count, the row-offset scans and k_rows_fill; the host read-back between them is not counted). */
 double grimb_engine_kernel_ms(const GrimbEngine* e, int which);
+
+/* ------------------------------------------------------------------------------------------
+ * Device-resident genotype interface: a genotype tensor in, ranked result rows out, both encoded and
+ * decoded on the device, so a caller holding typed genotypes in HBM needs neither the text pipeline nor
+ * the packed batch / GrimbCompact encodings.
+ * ------------------------------------------------------------------------------------------ */
+
+/* ids: DEVICE [n_subjects][L][2] allele ids in the tables' dictionary (id = position in the locus's sorted allele
+ * list + 1; side 0 = the allele written before the '+'), 4-byte aligned; 0/0 = locus untyped; ids past the table
+ * are subject-local names of alleles absent from it (n_l + 1, n_l + 2).  prior_index (DEVICE [S] or NULL) and
+ * priors (DEVICE [n_priors][P][P]) pass through to the batch.  type_allowed: HOST [1 << L] or NULL, as in
+ * GrimbTextDesc (Plan_A_Matrix).  A subject with one side of a locus 0, an id wider than its locus's key field,
+ * no typed locus, or (type_allowed) a typed-locus pattern that is no matrix row is skipped (GRIMB_ST_SKIPPED, no
+ * rows); the call does not fail for it.  *out gets a batch in buffers the engine owns (valid until the engine's
+ * next call of this function): the PACKED form when the build has 64-bit keys, L <= 5 and every subject is fully
+ * typed or skipped, else the general form (counts = NULL, allele_off by a device scan).  The call waits for one
+ * 16-byte read-back (which form applies, and the allele total) on `cuda_stream` (0 = engine stream). */
+int grimb_batch_from_genotypes(GrimbEngine* e, const uint16_t* ids, int64_t n_subjects, const uint32_t* prior_index,
+                               const double* priors, int32_t n_priors, const uint8_t* type_allowed, GrimbBatch* out,
+                               void* cuda_stream);
+
+/* Result rows of a finished device call (grimb_impute_device, or _async + finish), decoded on the device.  Every
+ * pointer is a DEVICE pointer except `totals`.  Per subject [S]: status, plans and the counts the reference prints
+ * (tot_umug, tot_pmug), flags (GRIMB_ROWS_*).  Four row kinds, each with its own offsets off[k] [S+1] and rows in
+ * rank order; a subject has rows only with status GRIMB_ST_OK, and only for the outputs the configuration enables:
+ *   GRIMB_ROWS_UMUG      rows[0] [n][L][2] per-locus allele pairs (min id, max id), 0/0 at an untyped locus
+ *   GRIMB_ROWS_PMUG      rows[1] [n][2][L] haplotype 1 then haplotype 2 in first-seen orientation, 0 = no allele
+ *   GRIMB_ROWS_UMUG_POPS rows[2] [n][2] population indices (0xFFFF = all_pops) as the kernels recorded them (the
+ *   GRIMB_ROWS_PMUG_POPS rows[3] [n][2]  .umug.pops text sorts the two names; these rows do not)
+ * prob[k] [n]: probabilities, copied bit for bit.  Table alleles keep their dictionary ids (id order = the
+ * reference's string order); an unknown allele keeps its subject-local id.  totals (HOST [4]) get the rows needed
+ * per kind; if one exceeds capacity[k] the call returns GRIMB_E_CAPACITY and writes no rows. */
+#define GRIMB_ROWS_UMUG 0
+#define GRIMB_ROWS_PMUG 1
+#define GRIMB_ROWS_UMUG_POPS 2
+#define GRIMB_ROWS_PMUG_POPS 3
+#define GRIMB_ROWS_HAS_RESULTS 1  /* flags bit 0: the subject has result rows                          */
+#define GRIMB_ROWS_MISS 2         /* flags bit 1: the reference writes the subject to .miss (OK status, haplotype
+                                     output on, no UMUG and no PMUG row; nothing when the haplotype output is off) */
+#define GRIMB_ROWS_PROBLEM 4      /* flags bit 2: .problem: SKIPPED, FAULT, or NO_PHASES with the haplotype output on */
+typedef struct {
+  uint8_t* status;              /* [S] GRIMB_ST_*                                                     */
+  uint8_t* plan_umug;           /* [S] GRIMB_PLAN_*                                                   */
+  uint8_t* plan_pmug;           /* [S]                                                                */
+  uint8_t* flags;               /* [S] GRIMB_ROWS_HAS_RESULTS | GRIMB_ROWS_MISS | GRIMB_ROWS_PROBLEM   */
+  uint32_t* tot_umug;           /* [S]                                                                */
+  uint32_t* tot_pmug;           /* [S]                                                                */
+  int64_t* off[4];              /* [S+1] per row kind                                                 */
+  uint16_t* rows[4];            /* per row kind, see above                                            */
+  double* prob[4];              /* [capacity[k]]                                                      */
+  int64_t capacity[4];          /* rows each kind's arrays hold                                       */
+  int64_t* totals;              /* HOST [4]: rows needed per kind                                     */
+} GrimbRows;
+
+/* cfg: the configuration of the call that produced `res`; batch: its batch (SIMPLE / TYPED rows take the
+ * subject's own alleles from it), any form; res: its GrimbResults (device arrays).  Synchronous on `cuda_stream`
+ * (0 = engine stream) for the 32-byte read-back of the totals. */
+int grimb_results_rows(GrimbEngine* e, const GrimbConfig* cfg, const GrimbBatch* batch, const GrimbResults* res,
+                       const GrimbRows* rows, void* cuda_stream);
 
 /* ------------------------------------------------------------------------------------------
  * Text pipeline (host C++, multi-threaded): the steps either side of the kernels.  Replaces the

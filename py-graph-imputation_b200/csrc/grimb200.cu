@@ -2821,6 +2821,13 @@ struct GrimbEngine {
   double last_worklist = -1; // subjects the last call handed from a warp-per-subject kernel to k_impute
   int typed_ctas = 0;        // resident CTAs of k_impute_typed on this device (0: P > 32, kernel unused)
   uint32_t typed_per_warp = 0;
+  // grimb_batch_from_genotypes (the batch it returns lives here) and grimb_results_rows; grow-only
+  DevBuf geno_keys, geno_flags, geno_mask, geno_off, geno_alleles, geno_small, scan_tmp;
+  unsigned long long* h_small = nullptr;   // pinned: the read-backs of both calls
+  cudaEvent_t ev_geno[4] = {nullptr, nullptr, nullptr, nullptr};   // [0,1] k_geno_encode, [2,3] scan + k_geno_fill
+  int ev_geno_valid = 0;                   // bit 0 / bit 1: pair recorded by the last call
+  cudaEvent_t ev_rows[4] = {nullptr, nullptr, nullptr, nullptr};   // [0,1] count + scans, [2,3] k_rows_fill
+  int ev_rows_valid = 0;
 };
 
 extern "C" int grimb_engine_free(GrimbEngine* e);
@@ -2918,6 +2925,9 @@ extern "C" int grimb_engine_create(const GrimbTables* t, int64_t workspace_bytes
   for (int i = 0; i < 2; ++i) CKE(cudaEventCreate(&e->ev_score[i]));
   for (int i = 0; i < 2; ++i) CKE(cudaEventCreate(&e->ev_slots[i]));
   CKE(cudaEventCreateWithFlags(&e->ev_done, cudaEventDisableTiming));
+  for (int i = 0; i < 4; ++i) CKE(cudaEventCreate(&e->ev_geno[i]));
+  for (int i = 0; i < 4; ++i) CKE(cudaEventCreate(&e->ev_rows[i]));
+  CKE(cudaMallocHost((void**)&e->h_small, 8 * sizeof(unsigned long long)));
   e->pre_max = 4096;
   if (const char* gs = getenv("GRIMB_GROUP_SUBJECTS")) {
     const long long v = atoll(gs);
@@ -2963,6 +2973,11 @@ extern "C" int grimb_engine_free(GrimbEngine* e) {
   for (int i = 0; i < 2; ++i)
     if (e->ev_slots[i]) cudaEventDestroy(e->ev_slots[i]);
   if (e->ev_done) cudaEventDestroy(e->ev_done);
+  for (int i = 0; i < 4; ++i) {
+    if (e->ev_geno[i]) cudaEventDestroy(e->ev_geno[i]);
+    if (e->ev_rows[i]) cudaEventDestroy(e->ev_rows[i]);
+  }
+  if (e->h_small) cudaFreeHost(e->h_small);
   if (e->h_gather) cudaFreeHost(e->h_gather);
   if (e->h_cnt) cudaFreeHost(e->h_cnt);
   if (e->h_tail) cudaFreeHost(e->h_tail);
@@ -2979,6 +2994,22 @@ extern "C" int64_t grimb_engine_launches(const GrimbEngine* e) { return e ? e->l
 extern "C" double grimb_engine_kernel_ms(const GrimbEngine* e, int which) {
   if (e && which == 3) return e->last_worklist;
   if (e && which == 6) return (double)e->last_probe;
+  if (e && (which == 7 || which == 8)) {   // sum of the event pairs the last grimb_batch_from_genotypes / _results_rows recorded
+    const cudaEvent_t* ev = which == 7 ? e->ev_geno : e->ev_rows;
+    const int valid = which == 7 ? e->ev_geno_valid : e->ev_rows_valid;
+    if (!valid) return -1.0;
+    double sum = 0.0;
+    for (int k = 0; k < 2; ++k) {
+      float ms = 0.f;
+      if (!(valid & (1 << k))) continue;
+      if (cudaEventElapsedTime(&ms, ev[2 * k], ev[2 * k + 1]) != cudaSuccess) {
+        cudaGetLastError();
+        return -1.0;
+      }
+      sum += ms;
+    }
+    return sum;
+  }
   if (e && which == 5) {   // k_impute_slots
     float ms5 = -1.f;
     if (!e->ev_slots_valid || cudaEventElapsedTime(&ms5, e->ev_slots[0], e->ev_slots[1]) != cudaSuccess) {
@@ -3577,4 +3608,442 @@ extern "C" int grimb_impute_host(GrimbEngine* e, const GrimbConfig* cfg, const G
   }
   e->last_worklist = wl;
   return totals_from(end, wl, r);
+}
+
+// ------------------------------------------------------------------------------------------
+// Device-resident genotype interface (include/grimb200.h): genotype tensor -> GrimbBatch, and the
+// results of a finished call -> ragged rows.  Integer work only; probabilities are copied as bits.
+// ------------------------------------------------------------------------------------------
+enum { GENO_PARTIAL = 0, GENO_ALLELES = 1 };   // geno_small counters: valid subjects typed at some loci only, allele ids
+
+// Small per-call parameters of k_geno_encode, in device memory (indexed per locus / pattern).
+struct GenoParams {
+  uint32_t allow[16];           // bit m: typed-locus pattern m is a Plan_A_Matrix row (all ones without a matrix)
+  uint32_t n_alleles[GRIMB_MAX_LOCI];
+  uint8_t shift[GRIMB_MAX_LOCI], width[GRIMB_MAX_LOCI];
+};
+
+// One thread per subject: validate, write typed_mask and the allele count (scanned into allele_off later),
+// and -- when the packed form may serve this build -- the two packed keys and the flag word.
+template <bool PACK>
+__global__ void __launch_bounds__(256) k_geno_encode(const uint32_t* __restrict__ ids, int64_t S, int L,
+                                                     const GenoParams* __restrict__ gp, uint16_t* __restrict__ typed_mask,
+                                                     uint32_t* __restrict__ count, uint64_t* __restrict__ keys,
+                                                     uint16_t* __restrict__ flags, unsigned long long* __restrict__ small) {
+  const int64_t s = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  uint32_t typed = 0;
+  if (s < S) {
+    uint32_t mask = 0;
+    bool bad = false;
+    uint64_t k0 = 0, k1 = 0;
+    uint32_t fl = 0;
+    const uint32_t* p = ids + s * L;
+    for (int l = 0; l < L; ++l) {
+      const uint32_t v = __ldg(p + l);
+      const uint32_t a0 = v & 0xFFFFu, a1 = v >> 16;
+      if ((a0 | a1) == 0u) continue;
+      const uint32_t sh = gp->shift[l], cap = (1u << gp->width[l]) - 1u;
+      if (a0 == 0u || a1 == 0u || a0 > cap || a1 > cap) bad = true;
+      mask |= 1u << l;
+      if (PACK) {
+        k0 |= (uint64_t)a0 << sh;
+        k1 |= (uint64_t)a1 << sh;
+        fl |= (a0 != a1 ? 1u : 0u) << l;
+        fl |= (a0 > gp->n_alleles[l] ? 1u : 0u) << (5 + l);
+        fl |= (a1 > gp->n_alleles[l] ? 1u : 0u) << (10 + l);
+      }
+    }
+    if (mask == 0u || !((gp->allow[mask >> 5] >> (mask & 31u)) & 1u)) bad = true;
+    typed = bad ? 0u : mask;
+    typed_mask[s] = (uint16_t)typed;
+    count[s] = 2u * (uint32_t)__popc(typed);
+    if (PACK) {
+      const bool full = typed == (1u << L) - 1u;
+      keys[2 * s] = full ? k0 : 0ull;
+      keys[2 * s + 1] = full ? k1 : 0ull;
+      flags[s] = (uint16_t)(full ? fl : 0x8000u);
+    }
+  }
+  // warp-aggregated counters: subjects the packed form cannot carry, allele ids of the general form
+  const bool partial = typed != 0u && typed != (1u << L) - 1u;
+  const unsigned int np = __popc(__ballot_sync(0xFFFFFFFFu, partial));
+  unsigned int na = 2u * (unsigned int)__popc(typed);
+  for (int o = 16; o > 0; o >>= 1) na += __shfl_xor_sync(0xFFFFFFFFu, na, o);
+  if ((threadIdx.x & 31u) == 0u) {
+    if (np) atomicAdd(small + GENO_PARTIAL, (unsigned long long)np);
+    if (na) atomicAdd(small + GENO_ALLELES, (unsigned long long)na);
+  }
+}
+
+// General form: the typed loci's ids, side 0 then side 1, at the subject's scanned offset.
+__global__ void __launch_bounds__(256) k_geno_fill(const uint32_t* __restrict__ ids, int64_t S, int L,
+                                                   const uint16_t* __restrict__ typed_mask, const uint32_t* __restrict__ off,
+                                                   uint16_t* __restrict__ alleles) {
+  const int64_t s = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (s >= S) return;
+  const uint32_t typed = typed_mask[s];
+  uint32_t o = off[s];
+  const uint32_t* p = ids + s * L;
+  for (int l = 0; l < L; ++l) {
+    if (!((typed >> l) & 1u)) continue;
+    const uint32_t v = __ldg(p + l);
+    alleles[o] = (uint16_t)(v & 0xFFFFu);
+    alleles[o + 1] = (uint16_t)(v >> 16);
+    o += 2;
+  }
+}
+
+extern "C" int grimb_batch_from_genotypes(GrimbEngine* e, const uint16_t* ids, int64_t n_subjects, const uint32_t* prior_index,
+                                          const double* priors, int32_t n_priors, const uint8_t* type_allowed, GrimbBatch* out,
+                                          void* cuda_stream) {
+  if (!e || !out || !priors || n_priors < 1) return fail(GRIMB_E_ARG, "null argument");
+  if (n_subjects < 0 || n_subjects > 0x7FFFFFF0ll) return fail(GRIMB_E_ARG, "bad n_subjects");
+  if (n_subjects > 0 && (!ids || ((uintptr_t)ids & 3u))) return fail(GRIMB_E_ARG, "ids must be a 4-byte aligned device array");
+  CK(cudaSetDevice(e->device));
+  const TablesView& tv = e->tables->view;
+  const int L = tv.L;
+  const int64_t S = n_subjects;
+  cudaStream_t st = cuda_stream ? (cudaStream_t)cuda_stream : e->stream;
+  GenoParams gp;
+  memset(&gp, 0, sizeof(gp));
+  for (uint32_t m = 0; m < (1u << L); ++m)
+    if (!type_allowed || type_allowed[m]) gp.allow[m >> 5] |= 1u << (m & 31u);
+  for (int l = 0; l < L; ++l) {
+    gp.n_alleles[l] = tv.n_alleles[l];
+    gp.shift[l] = tv.shift[l];
+    gp.width[l] = tv.width[l];
+  }
+  const bool packable = GRIMB_KW == 1 && L <= 5;
+  CK(e->geno_mask.reserve((size_t)S * 2 + 16));
+  CK(e->geno_off.reserve((size_t)(S + 1) * 4 + 16));
+  CK(e->geno_small.reserve(64 + sizeof(GenoParams)));
+  if (packable) {
+    CK(e->geno_keys.reserve((size_t)S * 16 + 16));
+    CK(e->geno_flags.reserve((size_t)S * 2 + 16));
+  }
+  unsigned long long* small = (unsigned long long*)e->geno_small.p;
+  GenoParams* d_gp = (GenoParams*)((char*)e->geno_small.p + 64);
+  CK(cudaMemsetAsync(small, 0, 64, st));
+  CK(cudaMemcpyAsync(d_gp, &gp, sizeof(gp), cudaMemcpyHostToDevice, st));
+  uint32_t* off = (uint32_t*)e->geno_off.p;
+  CK(cudaMemsetAsync(off + S, 0, 4, st));
+  e->ev_geno_valid = 0;
+  if (S > 0) {
+    if (e->timing) CK(cudaEventRecord(e->ev_geno[0], st));
+    const unsigned g = nblk((uint64_t)S);
+    if (packable)
+      k_geno_encode<true><<<g, 256, 0, st>>>((const uint32_t*)ids, S, L, d_gp, (uint16_t*)e->geno_mask.p, off,
+                                            (uint64_t*)e->geno_keys.p, (uint16_t*)e->geno_flags.p, small);
+    else
+      k_geno_encode<false><<<g, 256, 0, st>>>((const uint32_t*)ids, S, L, d_gp, (uint16_t*)e->geno_mask.p, off, nullptr, nullptr,
+                                             small);
+    CK(cudaGetLastError());
+    if (e->timing) CK(cudaEventRecord(e->ev_geno[1], st));
+    e->ev_geno_valid = e->timing ? 1 : 0;
+    e->launches += 1;
+  }
+  CK(cudaMemcpyAsync(e->h_small, small, 16, cudaMemcpyDeviceToHost, st));
+  CK(cudaStreamSynchronize(st));
+  const unsigned long long partial = e->h_small[GENO_PARTIAL], n_ids = e->h_small[GENO_ALLELES];
+  GrimbBatch b;
+  memset(&b, 0, sizeof(b));
+  b.n_subjects = S;
+  b.prior_index = prior_index;
+  b.priors = priors;
+  b.n_priors = n_priors;
+  if (packable && partial == 0) {
+    b.packed_keys = (const uint64_t*)e->geno_keys.p;
+    b.packed_flags = (const uint16_t*)e->geno_flags.p;
+    *out = b;
+    return GRIMB_OK;
+  }
+  if (n_ids > 0xFFFFFFF0ull) return fail(GRIMB_E_ARG, "more than 2^32 allele ids in one batch");
+  CK(e->geno_alleles.reserve((size_t)n_ids * 2 + 16));
+  if (S > 0) {
+    size_t tb = 0;
+    CK(cub::DeviceScan::ExclusiveSum(nullptr, tb, off, off, (int)(S + 1), st));
+    CK(e->scan_tmp.reserve(tb + 16));
+    if (e->timing) CK(cudaEventRecord(e->ev_geno[2], st));
+    CK(cub::DeviceScan::ExclusiveSum(e->scan_tmp.p, tb, off, off, (int)(S + 1), st));
+    k_geno_fill<<<nblk((uint64_t)S), 256, 0, st>>>((const uint32_t*)ids, S, L, (const uint16_t*)e->geno_mask.p, off,
+                                                  (uint16_t*)e->geno_alleles.p);
+    CK(cudaGetLastError());
+    if (e->timing) CK(cudaEventRecord(e->ev_geno[3], st));
+    e->ev_geno_valid |= e->timing ? 2 : 0;
+    e->launches += 2;
+  }
+  b.typed_mask = (const uint16_t*)e->geno_mask.p;
+  b.counts = nullptr;
+  b.allele_off = off;
+  b.alleles = (const uint16_t*)e->geno_alleles.p;
+  b.n_alleles_total = (int64_t)n_ids;
+  *out = b;
+  return GRIMB_OK;
+}
+
+// What the row decoder needs of the configuration, by value.
+struct RowsCfg {
+  int32_t L, out_u, out_p, n_results, n_pop_results;
+};
+
+// Per-subject view of a result record (GrimbCompact + its words or its GrimbSubjectResult), the one place
+// that reads the record layout of include/grimb200.h for the decoder.
+struct RowsRec {
+  uint32_t status, kind, has, n[4];        // rows per kind (GRIMB_ROWS_*), gated by status and configuration
+  uint32_t plan_u, plan_p, tot_u, tot_p;
+  uint32_t n_pm;                           // SIMPLE / TYPED: PMUG rows of the record
+  uint64_t phases;                         // SIMPLE: 4 bits per row; TYPED: the header (12 bits per row from bit 16)
+  const uint64_t* pm_prob;                 // SIMPLE / TYPED: PMUG probabilities (nullptr: `total`)
+  const uint64_t* pop_prob;                // TYPED: population-pair probabilities, then their codes
+  const uint64_t* pop_code;
+  double total;
+  const GrimbSubjectResult* g;             // GENERAL (nullptr: no record)
+};
+
+__device__ __forceinline__ RowsRec rows_record(const GrimbResults& R, const RowsCfg& c, uint64_t s) {
+  RowsRec r;
+  const GrimbCompact cp = R.compact[s];
+  r.status = cp.status;
+  r.kind = cp.kind_flags & 3u;
+  r.has = (cp.kind_flags & GRIMB_KIND_HAS_RESULTS) ? 1u : 0u;
+  r.total = cp.total;
+  r.g = nullptr;
+  r.pm_prob = r.pop_prob = r.pop_code = nullptr;
+  r.phases = 0;
+  r.n_pm = 0;
+  r.n[0] = r.n[1] = r.n[2] = r.n[3] = 0;
+  r.plan_u = r.plan_p = r.tot_u = r.tot_p = 0;
+  const bool ok = r.status == GRIMB_ST_OK;
+  if (r.kind == GRIMB_KIND_GENERAL) {
+    if (cp.off != 0xFFFFFFFFu && (int64_t)cp.off < R.general_capacity) {
+      r.g = R.general + cp.off;
+      const GrimbSubjectResult& g = *r.g;
+      r.plan_u = g.plan_umug;
+      r.plan_p = g.plan_pmug;
+      r.tot_u = g.tot_umug;
+      r.tot_p = g.tot_pmug;
+      if (ok) {
+        r.n[0] = c.out_u ? g.n_umug : 0u;
+        r.n[1] = c.out_p ? g.n_pmug : 0u;
+        r.n[2] = c.out_u ? g.n_umug_pops : 0u;
+        r.n[3] = c.out_p ? g.n_pmug_pops : 0u;
+      }
+    }
+    return r;
+  }
+  const uint64_t* w = R.words + cp.off;
+  uint32_t n_pm = cp.kind_flags >> 4, n_pops;
+  if (r.kind == GRIMB_KIND_SIMPLE && n_pm == 15u) {   // long form: a count word, a word of phase ids, the probabilities
+    n_pm = w[0] > 16u ? 16u : (uint32_t)w[0];
+    r.phases = w[1];
+    r.pm_prob = w + 2;
+    n_pops = (r.has && c.n_pop_results >= 1) ? 1u : 0u;
+  } else if (r.kind == GRIMB_KIND_SIMPLE) {
+    r.phases = cp.phases;
+    r.pm_prob = (cp.kind_flags & GRIMB_KIND_WORDS) ? w : nullptr;
+    n_pops = (r.has && c.n_pop_results >= 1) ? 1u : 0u;
+  } else {
+    r.phases = w[0];
+    n_pops = (uint32_t)(w[0] & 0xFFFFu);
+    r.pm_prob = w + 1;
+    r.pop_prob = w + 1 + n_pm;
+    r.pop_code = r.pop_prob + n_pops;
+  }
+  r.n_pm = n_pm;
+  r.plan_u = c.out_u ? GRIMB_PLAN_A : GRIMB_PLAN_NONE;
+  r.plan_p = c.out_p ? GRIMB_PLAN_A : GRIMB_PLAN_NONE;
+  r.tot_u = (r.has && c.out_u) ? 1u : 0u;
+  r.tot_p = c.out_p ? (r.has ? (n_pm > 1u ? n_pm : 1u) : 0u) : 0u;
+  if (ok) {
+    r.n[0] = (c.out_u && r.has && c.n_results >= 1) ? 1u : 0u;
+    r.n[1] = c.out_p ? n_pm : 0u;
+    r.n[2] = (c.out_u && r.has) ? n_pops : 0u;
+    r.n[3] = c.out_p ? n_pops : 0u;
+  }
+  return r;
+}
+
+__global__ void __launch_bounds__(256) k_rows_count(GrimbResults R, RowsCfg c, int64_t S, GrimbRows O) {
+  const int64_t s = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (s >= S) return;
+  const RowsRec r = rows_record(R, c, (uint64_t)s);
+  uint32_t fl = r.has ? GRIMB_ROWS_HAS_RESULTS : 0u;
+  if (r.status == GRIMB_ST_OK && c.out_p && r.tot_p == 0u && r.tot_u == 0u) fl |= GRIMB_ROWS_MISS;
+  if (r.status == GRIMB_ST_SKIPPED || r.status == GRIMB_ST_FAULT || (r.status == GRIMB_ST_NO_PHASES && c.out_p))
+    fl |= GRIMB_ROWS_PROBLEM;
+  O.status[s] = (uint8_t)r.status;
+  O.plan_umug[s] = (uint8_t)r.plan_u;
+  O.plan_pmug[s] = (uint8_t)r.plan_p;
+  O.flags[s] = (uint8_t)fl;
+  O.tot_umug[s] = r.tot_u;
+  O.tot_pmug[s] = r.tot_p;
+  for (int k = 0; k < 4; ++k) O.off[k][s] = (int64_t)r.n[k];
+}
+
+// the packed key of a hap row (GRIMB_KEY_WORDS little-endian words)
+__device__ __forceinline__ hkey row_key_a(const GrimbHapRow& h) {
+#if GRIMB_KW == 1
+  return h.a;
+#else
+  return (hkey)h.a[0] | ((hkey)h.a[1] << 64);
+#endif
+}
+__device__ __forceinline__ hkey row_key_b(const GrimbHapRow& h) {
+#if GRIMB_KW == 1
+  return h.b;
+#else
+  return (hkey)h.b[0] | ((hkey)h.b[1] << 64);
+#endif
+}
+
+__global__ void __launch_bounds__(256) k_rows_fill(GrimbResults R, RowsCfg c, int64_t S, GrimbBatch B, TablesView T, GrimbRows O) {
+  const int64_t s = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (s >= S) return;
+  const RowsRec r = rows_record(R, c, (uint64_t)s);
+  if ((r.n[0] | r.n[1] | r.n[2] | r.n[3]) == 0u) return;
+  const int L = c.L;
+  int64_t o[4];
+  for (int k = 0; k < 4; ++k) o[k] = O.off[k][s];
+  uint16_t* um = O.rows[GRIMB_ROWS_UMUG] + o[0] * 2 * L;
+  uint16_t* pm = O.rows[GRIMB_ROWS_PMUG] + o[1] * 2 * L;
+  double* ump = O.prob[GRIMB_ROWS_UMUG] + o[0];
+  double* pmp = O.prob[GRIMB_ROWS_PMUG] + o[1];
+  if (r.g) {
+    const GrimbSubjectResult& g = *r.g;
+    for (uint32_t q = 0; q < r.n[0]; ++q) {
+      const GrimbHapRow h = R.hap_rows[g.hap_off + q];
+      const hkey a = row_key_a(h), b = row_key_b(h);
+      for (int l = 0; l < L; ++l) {
+        const uint32_t x = (uint32_t)key_field(T, a, l), y = (uint32_t)key_field(T, b, l);
+        um[(q * L + l) * 2] = (uint16_t)(x < y ? x : y);
+        um[(q * L + l) * 2 + 1] = (uint16_t)(x < y ? y : x);
+      }
+      ump[q] = h.prob;
+    }
+    for (uint32_t q = 0; q < r.n[1]; ++q) {
+      const GrimbHapRow h = R.hap_rows[g.hap_off + g.n_umug + q];
+      const hkey a = row_key_a(h), b = row_key_b(h);
+      for (int l = 0; l < L; ++l) {
+        pm[(q * 2) * L + l] = (uint16_t)key_field(T, a, l);
+        pm[(q * 2 + 1) * L + l] = (uint16_t)key_field(T, b, l);
+      }
+      pmp[q] = h.prob;
+    }
+    for (int k = 2; k < 4; ++k) {
+      const uint64_t base = g.pop_off + (k == 3 ? g.n_umug_pops : 0u);
+      for (uint32_t q = 0; q < r.n[k]; ++q) {
+        const GrimbPopRow p = R.pop_rows[base + q];
+        O.rows[k][(o[k] + q) * 2] = p.pop_a;
+        O.rows[k][(o[k] + q) * 2 + 1] = p.pop_b;
+        O.prob[k][o[k] + q] = p.prob;
+      }
+    }
+    return;
+  }
+  // SIMPLE / TYPED: every locus typed with one allele per side; the rows follow from the subject's own alleles
+  hkey k0 = 0, k1 = 0;   // side-0 / side-1 alleles in the key layout (registers, not an indexed array)
+  if (B.packed_keys) {
+    k0 = (hkey)B.packed_keys[2 * s];
+    k1 = (hkey)B.packed_keys[2 * s + 1];
+  } else {
+    const uint16_t* a = B.alleles + B.allele_off[s];
+    for (int l = 0; l < L; ++l) {
+      k0 |= (hkey)a[2 * l] << T.shift[l];
+      k1 |= (hkey)a[2 * l + 1] << T.shift[l];
+    }
+  }
+  if (r.n[0]) {
+    for (int l = 0; l < L; ++l) {
+      const uint32_t x = (uint32_t)key_field(T, k0, l), y = (uint32_t)key_field(T, k1, l);
+      um[2 * l] = (uint16_t)(x < y ? x : y);
+      um[2 * l + 1] = (uint16_t)(x < y ? y : x);
+    }
+    ump[0] = r.total;
+  }
+  const bool typed = r.kind == GRIMB_KIND_TYPED;
+  for (uint32_t q = 0; q < r.n[1]; ++q) {
+    const uint32_t ph = typed ? (uint32_t)(r.phases >> (16 + 12 * q)) & 0xFFFu : (uint32_t)(r.phases >> (4 * q)) & 15u;
+    for (int l = 0; l < L; ++l) {
+      const uint32_t x = (uint32_t)key_field(T, k0, l), y = (uint32_t)key_field(T, k1, l);
+      const bool flip = (ph >> l) & 1u;
+      pm[(q * 2) * L + l] = (uint16_t)(flip ? y : x);
+      pm[(q * 2 + 1) * L + l] = (uint16_t)(flip ? x : y);
+    }
+    pmp[q] = r.pm_prob ? __longlong_as_double((long long)r.pm_prob[q]) : r.total;
+  }
+  for (int k = 2; k < 4; ++k) {
+    for (uint32_t q = 0; q < r.n[k]; ++q) {
+      uint32_t pa = 0, pb = 0;
+      double p = r.total;
+      if (r.pop_code) {
+        const uint32_t code = (uint32_t)(r.pop_code[q >> 2] >> (16 * (q & 3u))) & 0xFFFFu;
+        pa = code >> 8;
+        pb = code & 0xFFu;
+        p = __longlong_as_double((long long)r.pop_prob[q]);
+      }
+      O.rows[k][(o[k] + q) * 2] = (uint16_t)pa;
+      O.rows[k][(o[k] + q) * 2 + 1] = (uint16_t)pb;
+      O.prob[k][o[k] + q] = p;
+    }
+  }
+}
+
+extern "C" int grimb_results_rows(GrimbEngine* e, const GrimbConfig* cfg, const GrimbBatch* batch, const GrimbResults* res,
+                                  const GrimbRows* rows, void* cuda_stream) {
+  if (!e || !cfg || !batch || !res || !rows || !rows->totals) return fail(GRIMB_E_ARG, "null argument");
+  const int64_t S = batch->n_subjects;
+  if (S < 0 || S > 0x7FFFFFF0ll) return fail(GRIMB_E_ARG, "bad n_subjects");
+  for (int k = 0; k < 4; ++k)
+    if (!rows->off[k] || rows->capacity[k] < 0) return fail(GRIMB_E_ARG, "GrimbRows.off / capacity");
+  if (S > 0) {
+    if (!res->compact) return fail(GRIMB_E_ARG, "GrimbResults.compact missing");
+    if (!rows->status || !rows->plan_umug || !rows->plan_pmug || !rows->flags || !rows->tot_umug || !rows->tot_pmug)
+      return fail(GRIMB_E_ARG, "GrimbRows per-subject arrays missing");
+    if (!batch->packed_keys && (!batch->allele_off || !batch->alleles)) return fail(GRIMB_E_ARG, "batch arrays missing");
+  }
+  CK(cudaSetDevice(e->device));
+  cudaStream_t st = cuda_stream ? (cudaStream_t)cuda_stream : e->stream;
+  const TablesView& tv = e->tables->view;
+  RowsCfg c;
+  c.L = tv.L;
+  c.out_u = cfg->output_umug ? 1 : 0;
+  c.out_p = cfg->output_pmug ? 1 : 0;
+  c.n_results = cfg->n_results;
+  c.n_pop_results = cfg->n_pop_results;
+  e->ev_rows_valid = 0;
+  for (int k = 0; k < 4; ++k) CK(cudaMemsetAsync(rows->off[k] + S, 0, 8, st));
+  CK(e->geno_small.reserve(64 + sizeof(GenoParams)));
+  unsigned long long* small = (unsigned long long*)e->geno_small.p;
+  if (S > 0) {
+    size_t tb = 0;
+    CK(cub::DeviceScan::ExclusiveSum(nullptr, tb, rows->off[0], rows->off[0], (int)(S + 1), st));
+    CK(e->scan_tmp.reserve(tb + 16));
+    if (e->timing) CK(cudaEventRecord(e->ev_rows[0], st));
+    k_rows_count<<<nblk((uint64_t)S), 256, 0, st>>>(*res, c, S, *rows);
+    CK(cudaGetLastError());
+    for (int k = 0; k < 4; ++k) CK(cub::DeviceScan::ExclusiveSum(e->scan_tmp.p, tb, rows->off[k], rows->off[k], (int)(S + 1), st));
+    if (e->timing) CK(cudaEventRecord(e->ev_rows[1], st));
+    e->ev_rows_valid = e->timing ? 1 : 0;
+    e->launches += 5;
+  }
+  for (int k = 0; k < 4; ++k) CK(cudaMemcpyAsync(small + k, rows->off[k] + S, 8, cudaMemcpyDeviceToDevice, st));
+  CK(cudaMemcpyAsync(e->h_small, small, 32, cudaMemcpyDeviceToHost, st));
+  CK(cudaStreamSynchronize(st));
+  bool over = false;
+  for (int k = 0; k < 4; ++k) {
+    rows->totals[k] = (int64_t)e->h_small[k];
+    if (rows->totals[k] > rows->capacity[k]) over = true;
+    if (rows->totals[k] > 0 && (!rows->rows[k] || !rows->prob[k])) return fail(GRIMB_E_ARG, "GrimbRows row arrays missing");
+  }
+  if (over) return fail(GRIMB_E_CAPACITY, "row buffers too small (see GrimbRows.totals)");
+  if (S > 0 && (rows->totals[0] | rows->totals[1] | rows->totals[2] | rows->totals[3])) {
+    if (e->timing) CK(cudaEventRecord(e->ev_rows[2], st));
+    k_rows_fill<<<nblk((uint64_t)S), 256, 0, st>>>(*res, c, S, *batch, tv, *rows);
+    CK(cudaGetLastError());
+    if (e->timing) CK(cudaEventRecord(e->ev_rows[3], st));
+    e->ev_rows_valid |= e->timing ? 2 : 0;
+    e->launches += 1;
+  }
+  CK(cudaStreamSynchronize(st));
+  return GRIMB_OK;
 }

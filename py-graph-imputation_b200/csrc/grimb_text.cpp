@@ -1240,6 +1240,7 @@ extern "C" int64_t grimb_struct_size(int32_t which) {
     case 5: return (int64_t)sizeof(GrimbTextOut);
     case 6: return (int64_t)sizeof(GrimbFileStats);
     case 7: return (int64_t)sizeof(GrimbTableInfo);
+    case 8: return (int64_t)sizeof(GrimbRows);
     default: return -1;
   }
 }

@@ -158,6 +158,19 @@ class FileStats(C.Structure):
     ]
 
 
+class Rows(C.Structure):
+    """GrimbRows: ragged result rows decoded on the device (grimb_results_rows)."""
+    _fields_ = [
+        ("status", C.c_void_p), ("plan_umug", C.c_void_p), ("plan_pmug", C.c_void_p), ("flags", C.c_void_p),
+        ("tot_umug", C.c_void_p), ("tot_pmug", C.c_void_p),
+        ("off", C.c_void_p * 4), ("rows", C.c_void_p * 4), ("prob", C.c_void_p * 4), ("capacity", C.c_int64 * 4),
+        ("totals", C.c_void_p),
+    ]
+
+
+ROW_KINDS = ("umug", "pmug", "umug_pops", "pmug_pops")   # GRIMB_ROWS_* order
+ROWS_HAS_RESULTS, ROWS_MISS, ROWS_PROBLEM = 1, 2, 4
+
 OUT_KEYS = ("umug", "umug_pops", "pmug", "pmug_pops", "miss", "problem")  # GRIMB_OUT_* order
 
 _LIB = {}
@@ -225,11 +238,15 @@ def load(kw=1):
     lib.grimb_impute_file_sharded.argtypes = [C.c_void_p, C.POINTER(C.c_void_p), C.c_int32, C.POINTER(Config), C.c_char_p,
                                               C.POINTER(C.c_char_p), C.c_int64, C.c_int32, C.c_int32, C.c_char_p,
                                               C.POINTER(FileStats)]
+    lib.grimb_batch_from_genotypes.argtypes = [C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p, C.c_int32,
+                                               C.c_void_p, C.POINTER(Batch), C.c_void_p]
+    lib.grimb_results_rows.argtypes = [C.c_void_p, C.POINTER(Config), C.POINTER(Batch), C.POINTER(Results),
+                                       C.POINTER(Rows), C.c_void_p]
     if lib.grimb_abi_version() != 5:
         raise RuntimeError("libgrimb200.so ABI mismatch")
     lib.grimb_struct_size.argtypes = [C.c_int32]
     lib.grimb_struct_size.restype = C.c_int64
-    for which, ct in enumerate((Config, TableDesc, TextDesc, Batch, Results, TextOut, FileStats, TableInfo)):
+    for which, ct in enumerate((Config, TableDesc, TextDesc, Batch, Results, TextOut, FileStats, TableInfo, Rows)):
         if lib.grimb_struct_size(which) != C.sizeof(ct):
             raise RuntimeError("libgrimb200.so: layout of %s differs from the binding (%d vs %d bytes)"
                                % (ct.__name__, lib.grimb_struct_size(which), C.sizeof(ct)))
@@ -252,5 +269,5 @@ EXPORTED = [
     "grimb_impute_device", "grimb_impute_device_async", "grimb_impute_finish", "grimb_impute_host",
     "grimb_text_create", "grimb_text_free", "grimb_text_tokenise", "grimb_text_format", "grimb_impute_text",
     "grimb_impute_file", "grimb_file_count_lines", "grimb_file_write_at", "grimb_file_board_bytes",
-    "grimb_impute_file_sharded",
+    "grimb_impute_file_sharded", "grimb_batch_from_genotypes", "grimb_results_rows",
 ]

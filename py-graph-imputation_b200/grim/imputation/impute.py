@@ -634,6 +634,165 @@ class Imputation(object):
                 files["miss"].append(str(i) + "," + str(sid) + "\n")
             self._format_subject(sid, rows, files)
 
+    # ------------------------------------------------------------------ device-resident genotype interface
+    def prior_index(self, race1, race2):
+        """Index of the prior matrix for the race fields (race1, race2) of an input line (impute.py:1956-1975 of
+        the reference), for the prior_index argument of impute_genotypes."""
+        return self._prior_for(race1, race2)
+
+    def encode_genotypes(self, gl_strings):
+        """GL strings -> (ids uint16 [S][L][2] for impute_genotypes, unknown-name maps, text-path line indices).
+        ids[s, l] = the (side 0, side 1) allele ids of locus l (0/0: untyped); unknown[s] maps (locus, id) to the
+        name of an allele absent from the table, or is None.  A line with allele ambiguity, or one the tokeniser
+        classes as a problem or a fault, gets an all-zero row (it comes back SKIPPED) and its index is listed in
+        the third value: such lines belong on the text path (impute_text)."""
+        S, L = len(gl_strings), self.L
+        ids = np.zeros((S, L, 2), np.uint16)
+        unknown = [None] * S
+        text_path = []
+        for s, gl in enumerate(gl_strings):
+            hclass, payload = self._encode_gl(gl) if gl else (H_PROBLEM, None)
+            if hclass != H_OK or payload == "foreign" or (payload[1] > 1).any():
+                text_path.append(s)
+                continue
+            mask, _counts, flat, unknown[s] = payload
+            k = 0
+            for l in range(L):
+                if (mask >> l) & 1:
+                    ids[s, l] = flat[k:k + 2]
+                    k += 2
+        return ids, unknown, text_path
+
+    def _check_genotype_modes(self, em_mr, em):
+        if em_mr or self.cfg.hap_pop_pair:
+            raise NotImplementedError("impute_genotypes: the hap_pop_pair / em_mr output mode stays on the text path")
+        if em or self.cfg.em:
+            raise NotImplementedError("impute_genotypes: the em mode stays on the text path")
+        if self.cfg.encounter_order:
+            raise NotImplementedError("impute_genotypes: encounter_order (the impute_one seam) stays on impute_one")
+        if self.phase_masks is not None:
+            raise NotImplementedError("impute_genotypes: bin_imputation_in_file phase masks stay on the text path")
+
+    def impute_genotypes(self, ids, prior_index=None, em_mr=False, em=False):
+        """Imputes a batch of typed genotypes on the device: ids [S][L][2] allele ids as encode_genotypes returns
+        them (Graph.allele_id; 0/0 = untyped locus; ids past the table = subject-local unknown alleles), prior_index
+        [S] optional (Imputation.prior_index).  The batch is encoded, imputed and decoded on the GPU
+        (grimb_batch_from_genotypes, the imputation kernels, grimb_results_rows).  A CUDA torch tensor on the
+        table's device stays there and the results are CUDA tensors; a numpy array gives numpy results.
+        -> GenotypeResults.  Subjects that overflow a workspace tier are re-issued on the next one."""
+        import torch
+        self._check_genotype_modes(em_mr, em)
+        g = self.netGraph
+        dev = torch.device("cuda", g.device)
+        as_numpy = not isinstance(ids, torch.Tensor)
+        t = torch.from_numpy(np.ascontiguousarray(ids)) if as_numpy else ids
+        if t.dim() != 3 or t.shape[1] != self.L or t.shape[2] != 2:
+            raise ValueError("ids must be [S][%d][2]" % self.L)
+        if not as_numpy and (not t.is_cuda or t.device != dev):
+            raise ValueError("ids must be a numpy array or a CUDA tensor on the table's device (%s)" % dev)
+        t = t.view(torch.int16) if t.dtype in (torch.uint16, torch.int16) else t.to(torch.int32).to(torch.int16)
+        t = t.to(dev).contiguous()
+        S = int(t.shape[0])
+        pidx = self._prior_for(None, None)   # the matrix of a line without race fields (and priors never empty)
+        if prior_index is None:
+            pri = None if pidx == 0 else torch.full((S,), pidx, dtype=torch.int32, device=dev)
+        else:
+            pri = torch.as_tensor(np.asarray(prior_index) if not isinstance(prior_index, torch.Tensor) else prior_index)
+            if pri.shape != (S,) or (S and (int(pri.min()) < 0 or int(pri.max()) >= len(self._priors))):
+                raise ValueError("prior_index must be [S] indices from Imputation.prior_index")
+            pri = pri.to(device=dev, dtype=torch.int32).contiguous()
+        priors = torch.from_numpy(np.ascontiguousarray(np.stack(self._priors))).to(dev)
+        stream = torch.cuda.current_stream(dev)
+        self.cfg.hap_pop_pair = self.cfg.em = 0
+        out = None
+        todo = None   # indices of the subjects re-issued on this tier (None: the whole batch)
+        retries = 0
+        for tier in self.workspaces:
+            sub_ids = t if todo is None else t.index_select(0, todo).contiguous()
+            sub_pri = pri if (pri is None or todo is None) else pri.index_select(0, todo).contiguous()
+            part = self._genotype_pass(sub_ids, sub_pri, priors, tier, stream)
+            out = part if todo is None else _splice_rows(out, part, todo)
+            again = (part["status"] == _lib.ST_WORKSPACE).nonzero().flatten()
+            if again.numel() == 0:
+                break
+            todo = again if todo is None else todo.index_select(0, again)
+            retries += int(again.numel())
+        else:
+            raise MemoryError("a subject exceeds the largest workspace tier (GRIMB_WORKSPACES)")
+        self.stats["workspace_retries"] += retries
+        self.stats["subjects"] += S
+        if self.cfg.plan_a_only and self.cfg.planb and S:
+            st = out["status"] == _lib.ST_OK
+            left = st & (((out["tot_umug"] == 0) & bool(self.cfg.output_umug)) | ((out["tot_pmug"] == 0) & bool(self.cfg.output_pmug)))
+            if bool(left.any()):
+                s = int(left.nonzero()[0, 0])
+                raise NotImplementedError(
+                    "subject %d leaves Plan A without a result under a Plan_A_Matrix: the reference's Plan B is not "
+                    "well defined there; set \"planb\": false to write such subjects to the .miss file" % s)
+        return GenotypeResults(out, g.alleles, self.populations, retries, as_numpy)
+
+    def _genotype_pass(self, ids, pri, priors, tier, stream):
+        """One tier: encode, impute and decode `ids` (CUDA int16 [S][L][2]) -> dict of CUDA tensors."""
+        import torch
+        g, lib = self.netGraph, self.netGraph.lib
+        dev = ids.device
+        eng = g.engine(tier)
+        S, L = int(ids.shape[0]), self.L
+        sp = C.c_void_p(stream.cuda_stream)
+        b = _lib.Batch()
+        ta = self.type_allowed.ctypes.data if self.type_allowed is not None else None
+        _lib.check(lib.grimb_batch_from_genotypes(eng, ids.data_ptr(), S, pri.data_ptr() if pri is not None else None,
+                                                  priors.data_ptr(), priors.shape[0], ta, C.byref(b), sp),
+                   "grimb_batch_from_genotypes", lib)
+        hap_sz = 24 if g.kw == 1 else 40
+        caps = [S * 2 + 1024, S // 8 + 1024, S // 4 + 1024, S // 4 + 1024]
+        totals = np.zeros(9, np.int64)
+        while True:
+            compact = torch.empty(max(1, S) * 16, dtype=torch.uint8, device=dev)
+            bufs = [torch.empty(c * sz, dtype=torch.uint8, device=dev) for c, sz in zip(caps, (8, 48, hap_sz, 16))]
+            r = _lib.Results()
+            r.compact, r.totals = compact.data_ptr(), totals.ctypes.data
+            r.words, r.word_capacity = bufs[0].data_ptr(), caps[0]
+            r.general, r.general_capacity = bufs[1].data_ptr(), caps[1]
+            r.hap_rows, r.hap_capacity = bufs[2].data_ptr(), caps[2]
+            r.pop_rows, r.pop_capacity = bufs[3].data_ptr(), caps[3]
+            rc = lib.grimb_impute_device(eng, C.byref(self.cfg), C.byref(b), C.byref(r), sp)
+            if rc == _lib.E_CAPACITY:
+                caps = [max(c, int(x)) for c, x in zip(caps, totals[:4])]
+                continue
+            _lib.check(rc, "grimb_impute_device", lib)
+            break
+        out = {"status": torch.empty(S, dtype=torch.uint8, device=dev), "plan_umug": torch.empty(S, dtype=torch.uint8, device=dev),
+               "plan_pmug": torch.empty(S, dtype=torch.uint8, device=dev), "flags": torch.empty(S, dtype=torch.uint8, device=dev),
+               "tot_umug": torch.empty(S, dtype=torch.int32, device=dev), "tot_pmug": torch.empty(S, dtype=torch.int32, device=dev),
+               "pair_evals": int(totals[4])}
+        for k in _lib.ROW_KINDS:
+            out[k + "_off"] = torch.empty(S + 1, dtype=torch.int64, device=dev)
+        width = (2 * L, 2 * L, 2, 2)
+        rcap = list(getattr(self, "_row_caps", (S + 1024, 2 * S + 1024, S + 1024, S + 1024)))
+        rtot = np.zeros(4, np.int64)
+        while True:
+            rows = _lib.Rows()
+            for f in ("status", "plan_umug", "plan_pmug", "flags", "tot_umug", "tot_pmug"):
+                setattr(rows, f, out[f].data_ptr())
+            for i, k in enumerate(_lib.ROW_KINDS):
+                out[k] = torch.empty((rcap[i], width[i]), dtype=torch.int16, device=dev)
+                out[k + "_prob"] = torch.empty(rcap[i], dtype=torch.float64, device=dev)
+                rows.off[i], rows.rows[i], rows.prob[i] = out[k + "_off"].data_ptr(), out[k].data_ptr(), out[k + "_prob"].data_ptr()
+                rows.capacity[i] = rcap[i]
+            rows.totals = rtot.ctypes.data
+            rc = lib.grimb_results_rows(eng, C.byref(self.cfg), C.byref(b), C.byref(r), C.byref(rows), sp)
+            if rc == _lib.E_CAPACITY:
+                rcap = [max(c, int(x)) for c, x in zip(rcap, rtot)]
+                continue
+            _lib.check(rc, "grimb_results_rows", lib)
+            break
+        shapes = ((L, 2), (2, L), (2,), (2,))
+        for i, k in enumerate(_lib.ROW_KINDS):
+            out[k] = out[k][:int(rtot[i])].reshape((int(rtot[i]),) + shapes[i])
+            out[k + "_prob"] = out[k + "_prob"][:int(rtot[i])]
+        return out
+
     # ------------------------------------------------------------------ EM helpers (host only)
     # open_gl_string / open_phases_for_em (impute.py:305-351 of the reference) are list-building
     # utilities the EM driver calls around imputation; they involve no frequency lookup, so they are
@@ -896,3 +1055,70 @@ class Imputation(object):
         for k, ck in targets.items():
             with open(config[ck], "w") as f:
                 f.writelines(files[k])
+
+
+_SUBJECT_FIELDS = ("status", "plan_umug", "plan_pmug", "flags", "tot_umug", "tot_pmug")
+
+
+def _splice_rows(base, part, idx):
+    """Rows of the whole batch with the subjects `idx` (CUDA int64) taken from `part` (their re-issue)."""
+    import torch
+    out = {"pair_evals": base["pair_evals"] + part["pair_evals"]}
+    for f in _SUBJECT_FIELDS:
+        out[f] = base[f].clone()
+        out[f][idx] = part[f]
+    S, dev = base["status"].shape[0], base["status"].device
+    pos = torch.full((S,), -1, dtype=torch.int64, device=dev)
+    pos[idx] = torch.arange(idx.numel(), device=dev)
+    for k in _lib.ROW_KINDS:
+        bo, po = base[k + "_off"], part[k + "_off"]
+        cnt = bo[1:] - bo[:-1]
+        cnt[idx] = po[1:] - po[:-1]
+        off = torch.zeros(S + 1, dtype=torch.int64, device=dev)
+        torch.cumsum(cnt, 0, out=off[1:])
+        total = int(off[-1])
+        owner = torch.repeat_interleave(torch.arange(S, device=dev), cnt, output_size=total)
+        within = torch.arange(total, device=dev) - off[owner]
+        p = pos[owner]
+        mine = p >= 0
+        rows = torch.empty((total,) + tuple(base[k].shape[1:]), dtype=base[k].dtype, device=dev)
+        prob = torch.empty(total, dtype=torch.float64, device=dev)
+        src = po[p[mine]] + within[mine]
+        rows[mine], prob[mine] = part[k][src], part[k + "_prob"][src]
+        src = bo[owner[~mine]] + within[~mine]
+        rows[~mine], prob[~mine] = base[k][src], base[k + "_prob"][src]
+        out[k], out[k + "_prob"], out[k + "_off"] = rows, prob, off
+    return out
+
+
+class GenotypeResults(object):
+    """Result of Imputation.impute_genotypes: ragged rows in input order (include/grimb200.h, GrimbRows).
+
+    Per subject [S]: status (GRIMB_ST_*), plan_umug, plan_pmug (GRIMB_PLAN_*), tot_umug, tot_pmug (the counts the
+    reference prints), flags (bit 0 has results, bit 1 written to .miss, bit 2 written to .problem).
+    Per row kind k in ("umug", "pmug", "umug_pops", "pmug_pops"): k_off [S+1] (int64; subject s owns rows
+    k_off[s]:k_off[s+1], in rank order), k (uint16 rows: umug [n][L][2] (min id, max id) allele pairs, pmug [n][2][L]
+    haplotype 1 / haplotype 2 (0 = no allele), pop kinds [n][2] population indices, 0xFFFF = all_pops) and k_prob
+    [n] (float64).  alleles[l][id - 1] names table allele `id` of locus l; populations[p] names population p.
+    pair_evals: pair evaluations of the batch; workspace_retries: subjects re-issued on a bigger workspace tier.
+    Arrays are CUDA tensors when the input was one, numpy arrays otherwise."""
+
+    def __init__(self, d, alleles, populations, workspace_retries, as_numpy):
+        import torch
+        self.alleles, self.populations = alleles, populations
+        self.pair_evals, self.workspace_retries = d["pair_evals"], workspace_retries
+        for f in _SUBJECT_FIELDS:
+            v = d[f]   # uint8, or int32 storage of the uint32 totals
+            if as_numpy:
+                v = v.cpu().numpy()
+                setattr(self, f, v.view(np.uint32) if v.dtype == np.int32 else v)
+            else:
+                setattr(self, f, v.view(torch.uint32) if v.dtype == torch.int32 else v)
+        for k in _lib.ROW_KINDS:
+            rows = d[k]
+            setattr(self, k, rows.cpu().numpy().view(np.uint16) if as_numpy else rows.view(torch.uint16))
+            setattr(self, k + "_prob", d[k + "_prob"].cpu().numpy() if as_numpy else d[k + "_prob"])
+            setattr(self, k + "_off", d[k + "_off"].cpu().numpy() if as_numpy else d[k + "_off"])
+
+    def __len__(self):
+        return int(self.status.shape[0])
