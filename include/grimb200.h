@@ -308,7 +308,9 @@ int64_t grimb_engine_launches(const GrimbEngine* e);
  * 2 the two-level k_fast_probe2 (packed batch), 1 k_fast_probe on a packed batch, 0 k_fast_probe on
  * the general batch form, -1 none yet.  which = 7: the last grimb_batch_from_genotypes (k_geno_encode, plus the
  * allele-offset scan and k_geno_fill when it built the general form); which = 8: the last grimb_results_rows
- * (k_rows_count, the row-offset scans and k_rows_fill; the host read-back between them is not counted). */
+ * (k_rows_count, the row-offset scans and k_rows_fill; the host read-back between them is not counted); which = 9:
+ * the last grimb_batch_from_genotype_lists (k_gl_count and the input-offset scan, then k_gl_dedup, the
+ * allele-offset scan and k_gl_fill; the read-back between them is not counted). */
 double grimb_engine_kernel_ms(const GrimbEngine* e, int which);
 
 /* ------------------------------------------------------------------------------------------
@@ -331,6 +333,25 @@ int grimb_batch_from_genotypes(GrimbEngine* e, const uint16_t* ids, int64_t n_su
                                const double* priors, int32_t n_priors, const uint8_t* type_allowed, GrimbBatch* out,
                                void* cuda_stream);
 
+/* The same for subjects with allele ambiguity: ragged allele lists in, always the general batch form out.
+ * counts: DEVICE [n_subjects][L][2], the number of ids listed on side x of locus l (0/0 = locus untyped);
+ * alleles: DEVICE [n_alleles], the ids concatenated subject-major, locus ascending, side 0 then side 1, each list in
+ * the order it was written (the layout of GrimbBatch.alleles); ids as in grimb_batch_from_genotypes.  phase_mask
+ * (DEVICE [S] or NULL) passes through to GrimbBatch.phase_mask; prior_index, priors and type_allowed as above.
+ * A repeated id inside one side's list is dropped, the first occurrence kept (as the text tokenisers do).  A
+ * subject with exactly one side of a locus listing nothing, an id 0, an id wider than its locus's key field, no
+ * typed locus, or (type_allowed) a typed-locus pattern that is no matrix row is skipped (GRIMB_ST_SKIPPED, no rows).
+ * If the counts sum to anything but n_alleles the call returns GRIMB_E_ARG: it reads the counts first and checks
+ * their sum (one read-back) before any kernel reads `alleles`.  *out gets the general form with de-duplicated
+ * counts (non-NULL), allele_off and compacted alleles, in buffers the engine owns (valid until the engine's next
+ * call of this function); subjects with one allele per side at every locus still take the warp-per-subject kernels
+ * when no phase mask and no hap_pop_pair apply.  The call waits for two small read-backs on `cuda_stream`
+ * (0 = engine stream): the input total, then the de-duplicated total (n_alleles_total). */
+int grimb_batch_from_genotype_lists(GrimbEngine* e, const uint16_t* counts, const uint16_t* alleles, int64_t n_alleles,
+                                    int64_t n_subjects, const uint32_t* prior_index, const double* priors, int32_t n_priors,
+                                    const uint16_t* phase_mask, const uint8_t* type_allowed, GrimbBatch* out,
+                                    void* cuda_stream);
+
 /* Result rows of a finished device call (grimb_impute_device, or _async + finish), decoded on the device.  Every
  * pointer is a DEVICE pointer except `totals`.  Per subject [S]: status, plans and the counts the reference prints
  * (tot_umug, tot_pmug), flags (GRIMB_ROWS_*).  Four row kinds, each with its own offsets off[k] [S+1] and rows in
@@ -341,7 +362,10 @@ int grimb_batch_from_genotypes(GrimbEngine* e, const uint16_t* ids, int64_t n_su
  *   GRIMB_ROWS_PMUG_POPS rows[3] [n][2]  .umug.pops text sorts the two names; these rows do not)
  * prob[k] [n]: probabilities, copied bit for bit.  Table alleles keep their dictionary ids (id order = the
  * reference's string order); an unknown allele keeps its subject-local id.  totals (HOST [4]) get the rows needed
- * per kind; if one exceeds capacity[k] the call returns GRIMB_E_CAPACITY and writes no rows. */
+ * per kind; if one exceeds capacity[k] the call returns GRIMB_E_CAPACITY and writes no rows.  Under
+ * cfg->hap_pop_pair, pmug_pairs [capacity[GRIMB_ROWS_PMUG]][2] gets the populations of haplotype 1 and haplotype 2
+ * of each PMUG row (its companion pop row, see GrimbConfig.hap_pop_pair); it is then required
+ * (NULL: GRIMB_E_ARG) and ignored otherwise. */
 #define GRIMB_ROWS_UMUG 0
 #define GRIMB_ROWS_PMUG 1
 #define GRIMB_ROWS_UMUG_POPS 2
@@ -362,6 +386,7 @@ typedef struct {
   double* prob[4];              /* [capacity[k]]                                                      */
   int64_t capacity[4];          /* rows each kind's arrays hold                                       */
   int64_t* totals;              /* HOST [4]: rows needed per kind                                     */
+  uint16_t* pmug_pairs;         /* [capacity[GRIMB_ROWS_PMUG]][2] under hap_pop_pair, else unused     */
 } GrimbRows;
 
 /* cfg: the configuration of the call that produced `res`; batch: its batch (SIMPLE / TYPED rows take the

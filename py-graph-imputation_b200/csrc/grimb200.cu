@@ -2828,6 +2828,10 @@ struct GrimbEngine {
   int ev_geno_valid = 0;                   // bit 0 / bit 1: pair recorded by the last call
   cudaEvent_t ev_rows[4] = {nullptr, nullptr, nullptr, nullptr};   // [0,1] count + scans, [2,3] k_rows_fill
   int ev_rows_valid = 0;
+  // grimb_batch_from_genotype_lists (the batch it returns lives here); grow-only
+  DevBuf gl_in_off, gl_stage, gl_mask, gl_counts, gl_off, gl_alleles;
+  cudaEvent_t ev_gl[4] = {nullptr, nullptr, nullptr, nullptr};     // [0,1] k_gl_count + scan, [2,3] dedup, scan, fill
+  int ev_gl_valid = 0;
 };
 
 extern "C" int grimb_engine_free(GrimbEngine* e);
@@ -2927,6 +2931,7 @@ extern "C" int grimb_engine_create(const GrimbTables* t, int64_t workspace_bytes
   CKE(cudaEventCreateWithFlags(&e->ev_done, cudaEventDisableTiming));
   for (int i = 0; i < 4; ++i) CKE(cudaEventCreate(&e->ev_geno[i]));
   for (int i = 0; i < 4; ++i) CKE(cudaEventCreate(&e->ev_rows[i]));
+  for (int i = 0; i < 4; ++i) CKE(cudaEventCreate(&e->ev_gl[i]));
   CKE(cudaMallocHost((void**)&e->h_small, 8 * sizeof(unsigned long long)));
   e->pre_max = 4096;
   if (const char* gs = getenv("GRIMB_GROUP_SUBJECTS")) {
@@ -2976,6 +2981,7 @@ extern "C" int grimb_engine_free(GrimbEngine* e) {
   for (int i = 0; i < 4; ++i) {
     if (e->ev_geno[i]) cudaEventDestroy(e->ev_geno[i]);
     if (e->ev_rows[i]) cudaEventDestroy(e->ev_rows[i]);
+    if (e->ev_gl[i]) cudaEventDestroy(e->ev_gl[i]);
   }
   if (e->h_small) cudaFreeHost(e->h_small);
   if (e->h_gather) cudaFreeHost(e->h_gather);
@@ -2994,9 +3000,10 @@ extern "C" int64_t grimb_engine_launches(const GrimbEngine* e) { return e ? e->l
 extern "C" double grimb_engine_kernel_ms(const GrimbEngine* e, int which) {
   if (e && which == 3) return e->last_worklist;
   if (e && which == 6) return (double)e->last_probe;
-  if (e && (which == 7 || which == 8)) {   // sum of the event pairs the last grimb_batch_from_genotypes / _results_rows recorded
-    const cudaEvent_t* ev = which == 7 ? e->ev_geno : e->ev_rows;
-    const int valid = which == 7 ? e->ev_geno_valid : e->ev_rows_valid;
+  if (e && which >= 7 && which <= 9) {   // sum of the event pairs the last grimb_batch_from_genotypes / _results_rows /
+                                          // grimb_batch_from_genotype_lists recorded
+    const cudaEvent_t* ev = which == 7 ? e->ev_geno : which == 8 ? e->ev_rows : e->ev_gl;
+    const int valid = which == 7 ? e->ev_geno_valid : which == 8 ? e->ev_rows_valid : e->ev_gl_valid;
     if (!valid) return -1.0;
     double sum = 0.0;
     for (int k = 0; k < 2; ++k) {
@@ -3623,6 +3630,32 @@ struct GenoParams {
   uint8_t shift[GRIMB_MAX_LOCI], width[GRIMB_MAX_LOCI];
 };
 
+// Per-locus validation of both genotype encoders.  n0 / n1: ids listed on side 0 / side 1; lo / hi: the smallest /
+// largest of them; cap: the largest id the locus's key field holds.  Both sides empty = untyped; exactly one side
+// empty, an id 0 or an id wider than the key field = a bad subject (GRIMB_ST_SKIPPED).
+enum { GENO_UNTYPED = 0, GENO_TYPED = 1, GENO_BAD = 2 };
+__device__ __forceinline__ int geno_locus(uint32_t n0, uint32_t n1, uint32_t lo, uint32_t hi, uint32_t cap) {
+  if ((n0 | n1) == 0u) return GENO_UNTYPED;
+  return (n0 == 0u || n1 == 0u || lo == 0u || hi > cap) ? GENO_BAD : GENO_TYPED;
+}
+// The subject's typed-locus pattern: at least one locus, and a Plan_A_Matrix row when a matrix is in force.
+__device__ __forceinline__ bool geno_pattern_ok(const GenoParams* gp, uint32_t mask) {
+  return mask != 0u && ((gp->allow[mask >> 5] >> (mask & 31u)) & 1u);
+}
+
+static GenoParams geno_params(const TablesView& tv, const uint8_t* type_allowed) {
+  GenoParams gp;
+  memset(&gp, 0, sizeof(gp));
+  for (uint32_t m = 0; m < (1u << tv.L); ++m)
+    if (!type_allowed || type_allowed[m]) gp.allow[m >> 5] |= 1u << (m & 31u);
+  for (int l = 0; l < tv.L; ++l) {
+    gp.n_alleles[l] = tv.n_alleles[l];
+    gp.shift[l] = tv.shift[l];
+    gp.width[l] = tv.width[l];
+  }
+  return gp;
+}
+
 // One thread per subject: validate, write typed_mask and the allele count (scanned into allele_off later),
 // and -- when the packed form may serve this build -- the two packed keys and the flag word.
 template <bool PACK>
@@ -3641,9 +3674,10 @@ __global__ void __launch_bounds__(256) k_geno_encode(const uint32_t* __restrict_
     for (int l = 0; l < L; ++l) {
       const uint32_t v = __ldg(p + l);
       const uint32_t a0 = v & 0xFFFFu, a1 = v >> 16;
-      if ((a0 | a1) == 0u) continue;
       const uint32_t sh = gp->shift[l], cap = (1u << gp->width[l]) - 1u;
-      if (a0 == 0u || a1 == 0u || a0 > cap || a1 > cap) bad = true;
+      const int st = geno_locus(a0 != 0u, a1 != 0u, min(a0, a1), max(a0, a1), cap);
+      if (st == GENO_UNTYPED) continue;
+      if (st == GENO_BAD) bad = true;
       mask |= 1u << l;
       if (PACK) {
         k0 |= (uint64_t)a0 << sh;
@@ -3653,7 +3687,7 @@ __global__ void __launch_bounds__(256) k_geno_encode(const uint32_t* __restrict_
         fl |= (a1 > gp->n_alleles[l] ? 1u : 0u) << (10 + l);
       }
     }
-    if (mask == 0u || !((gp->allow[mask >> 5] >> (mask & 31u)) & 1u)) bad = true;
+    if (!geno_pattern_ok(gp, mask)) bad = true;
     typed = bad ? 0u : mask;
     typed_mask[s] = (uint16_t)typed;
     count[s] = 2u * (uint32_t)__popc(typed);
@@ -3704,15 +3738,7 @@ extern "C" int grimb_batch_from_genotypes(GrimbEngine* e, const uint16_t* ids, i
   const int L = tv.L;
   const int64_t S = n_subjects;
   cudaStream_t st = cuda_stream ? (cudaStream_t)cuda_stream : e->stream;
-  GenoParams gp;
-  memset(&gp, 0, sizeof(gp));
-  for (uint32_t m = 0; m < (1u << L); ++m)
-    if (!type_allowed || type_allowed[m]) gp.allow[m >> 5] |= 1u << (m & 31u);
-  for (int l = 0; l < L; ++l) {
-    gp.n_alleles[l] = tv.n_alleles[l];
-    gp.shift[l] = tv.shift[l];
-    gp.width[l] = tv.width[l];
-  }
+  const GenoParams gp = geno_params(tv, type_allowed);
   const bool packable = GRIMB_KW == 1 && L <= 5;
   CK(e->geno_mask.reserve((size_t)S * 2 + 16));
   CK(e->geno_off.reserve((size_t)(S + 1) * 4 + 16));
@@ -3781,9 +3807,161 @@ extern "C" int grimb_batch_from_genotypes(GrimbEngine* e, const uint16_t* ids, i
   return GRIMB_OK;
 }
 
+// ---- ragged allele lists (grimb_batch_from_genotype_lists) ----
+
+// One thread per subject: the number of ids the subject lists, i.e. its share of the caller's `alleles` (64-bit, so
+// that no sum of counts can wrap onto the caller's n_alleles); scanned into the input offsets.
+__global__ void __launch_bounds__(256) k_gl_count(const uint16_t* __restrict__ counts, int64_t S, int L,
+                                                  unsigned long long* __restrict__ in_off) {
+  const int64_t s = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (s >= S) return;
+  const uint16_t* c = counts + s * 2 * L;
+  unsigned long long n = 0;
+  for (int i = 0; i < 2 * L; ++i) n += __ldg(c + i);
+  in_off[s] = n;
+}
+
+// One thread per subject: validate (geno_locus, geno_pattern_ok), drop repeated ids of each side's list (the first
+// occurrence stays, as the host tokenisers do), and write the kept ids to `stage` at the subject's input offset,
+// the de-duplicated counts, the typed mask and the subject's kept total (scanned into allele_off next).  A bad
+// subject gets typed mask 0, counts 0 and total 0.  Lists may be long (40+ ids on a side): the repeat test walks
+// the side's earlier ids in the input, no fixed-size table.
+__global__ void __launch_bounds__(256) k_gl_dedup(const uint16_t* __restrict__ counts, const uint16_t* __restrict__ alleles,
+                                                  const unsigned long long* __restrict__ in_off, int64_t S, int L,
+                                                  const GenoParams* __restrict__ gp, uint16_t* __restrict__ stage,
+                                                  uint16_t* __restrict__ typed_mask, uint16_t* __restrict__ dcounts,
+                                                  uint32_t* __restrict__ dtot) {
+  const int64_t s = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (s >= S) return;
+  const uint16_t* c = counts + s * 2 * L;
+  uint16_t* dc = dcounts + s * 2 * L;
+  const unsigned long long base = in_off[s];
+  const uint16_t* src = alleles + base;
+  uint16_t* dst = stage + base;
+  uint32_t pos = 0, kept = 0, mask = 0;
+  bool bad = false;
+  for (int l = 0; l < L; ++l) {
+    const uint32_t n0 = __ldg(c + 2 * l), n1 = __ldg(c + 2 * l + 1);
+    uint32_t lo = 0xFFFFu, hi = 0u;
+    for (int x = 0; x < 2; ++x) {
+      const uint32_t n = x ? n1 : n0, first = pos;
+      uint32_t k = 0;
+      for (; pos < first + n; ++pos) {
+        const uint32_t v = __ldg(src + pos);
+        lo = min(lo, v);
+        hi = max(hi, v);
+        bool dup = false;
+        for (uint32_t j = first; j < pos && !dup; ++j) dup = __ldg(src + j) == v;
+        if (!dup) dst[kept + k++] = (uint16_t)v;
+      }
+      dc[2 * l + x] = (uint16_t)k;
+      kept += k;
+    }
+    const int st = geno_locus(n0, n1, lo, hi, (1u << gp->width[l]) - 1u);
+    if (st == GENO_BAD) bad = true;
+    if (st != GENO_UNTYPED) mask |= 1u << l;
+  }
+  if (!geno_pattern_ok(gp, mask)) bad = true;
+  if (bad) {
+    for (int i = 0; i < 2 * L; ++i) dc[i] = 0;
+    mask = kept = 0;
+  }
+  typed_mask[s] = (uint16_t)mask;
+  dtot[s] = kept;
+}
+
+// One thread per subject: the kept ids from the subject's input offset to its de-duplicated offset.
+__global__ void __launch_bounds__(256) k_gl_fill(const uint16_t* __restrict__ stage, const unsigned long long* __restrict__ in_off,
+                                                 const uint32_t* __restrict__ off, int64_t S, uint16_t* __restrict__ alleles) {
+  const int64_t s = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (s >= S) return;
+  const uint16_t* src = stage + in_off[s];
+  const uint32_t o = off[s], n = off[s + 1] - o;
+  for (uint32_t i = 0; i < n; ++i) alleles[o + i] = src[i];
+}
+
+extern "C" int grimb_batch_from_genotype_lists(GrimbEngine* e, const uint16_t* counts, const uint16_t* alleles, int64_t n_alleles,
+                                               int64_t n_subjects, const uint32_t* prior_index, const double* priors,
+                                               int32_t n_priors, const uint16_t* phase_mask, const uint8_t* type_allowed,
+                                               GrimbBatch* out, void* cuda_stream) {
+  if (!e || !out || !priors || n_priors < 1) return fail(GRIMB_E_ARG, "null argument");
+  if (n_subjects < 0 || n_subjects > 0x7FFFFFF0ll) return fail(GRIMB_E_ARG, "bad n_subjects");
+  if (n_alleles < 0 || n_alleles > 0xFFFFFFF0ll) return fail(GRIMB_E_ARG, "bad n_alleles (at most 2^32 - 16 ids)");
+  if (n_subjects > 0 && !counts) return fail(GRIMB_E_ARG, "counts missing");
+  if (n_alleles > 0 && !alleles) return fail(GRIMB_E_ARG, "alleles missing");
+  CK(cudaSetDevice(e->device));
+  const TablesView& tv = e->tables->view;
+  const int L = tv.L;
+  const int64_t S = n_subjects;
+  cudaStream_t st = cuda_stream ? (cudaStream_t)cuda_stream : e->stream;
+  const GenoParams gp = geno_params(tv, type_allowed);
+  CK(e->gl_in_off.reserve((size_t)(S + 1) * 8 + 16));
+  CK(e->gl_mask.reserve((size_t)S * 2 + 16));
+  CK(e->gl_counts.reserve((size_t)S * L * 4 + 16));
+  CK(e->gl_off.reserve((size_t)(S + 1) * 4 + 16));
+  CK(e->geno_small.reserve(64 + sizeof(GenoParams)));
+  unsigned long long* small = (unsigned long long*)e->geno_small.p;
+  GenoParams* d_gp = (GenoParams*)((char*)e->geno_small.p + 64);
+  unsigned long long* in_off = (unsigned long long*)e->gl_in_off.p;
+  uint32_t* off = (uint32_t*)e->gl_off.p;
+  CK(cudaMemcpyAsync(d_gp, &gp, sizeof(gp), cudaMemcpyHostToDevice, st));
+  CK(cudaMemsetAsync(in_off + S, 0, 8, st));
+  CK(cudaMemsetAsync(off + S, 0, 4, st));
+  e->ev_gl_valid = 0;
+  // pass 1 reads the counts only: the caller's lengths are checked before any kernel reads `alleles`
+  size_t tb = 0, tb32 = 0;
+  if (S > 0) {
+    CK(cub::DeviceScan::ExclusiveSum(nullptr, tb, in_off, in_off, (int)(S + 1), st));
+    CK(cub::DeviceScan::ExclusiveSum(nullptr, tb32, off, off, (int)(S + 1), st));
+    CK(e->scan_tmp.reserve((tb > tb32 ? tb : tb32) + 16));
+    if (e->timing) CK(cudaEventRecord(e->ev_gl[0], st));
+    k_gl_count<<<nblk((uint64_t)S), 256, 0, st>>>(counts, S, L, in_off);
+    CK(cudaGetLastError());
+    CK(cub::DeviceScan::ExclusiveSum(e->scan_tmp.p, tb, in_off, in_off, (int)(S + 1), st));
+    if (e->timing) CK(cudaEventRecord(e->ev_gl[1], st));
+    e->ev_gl_valid = e->timing ? 1 : 0;
+    e->launches += 2;
+  }
+  CK(cudaMemcpyAsync(e->h_small, in_off + S, 8, cudaMemcpyDeviceToHost, st));
+  CK(cudaStreamSynchronize(st));
+  if ((long long)e->h_small[0] != n_alleles || e->h_small[0] > 0xFFFFFFF0ull)
+    return fail(GRIMB_E_ARG, "the counts list a different number of ids than n_alleles");
+  CK(e->gl_stage.reserve((size_t)n_alleles * 2 + 16));
+  CK(e->gl_alleles.reserve((size_t)n_alleles * 2 + 16));
+  if (S > 0) {
+    if (e->timing) CK(cudaEventRecord(e->ev_gl[2], st));
+    k_gl_dedup<<<nblk((uint64_t)S), 256, 0, st>>>(counts, alleles, in_off, S, L, d_gp, (uint16_t*)e->gl_stage.p,
+                                                 (uint16_t*)e->gl_mask.p, (uint16_t*)e->gl_counts.p, off);
+    CK(cudaGetLastError());
+    CK(cub::DeviceScan::ExclusiveSum(e->scan_tmp.p, tb32, off, off, (int)(S + 1), st));
+    k_gl_fill<<<nblk((uint64_t)S), 256, 0, st>>>((const uint16_t*)e->gl_stage.p, in_off, off, S, (uint16_t*)e->gl_alleles.p);
+    CK(cudaGetLastError());
+    if (e->timing) CK(cudaEventRecord(e->ev_gl[3], st));
+    e->ev_gl_valid |= e->timing ? 2 : 0;
+    e->launches += 3;
+  }
+  // the de-duplicated total, for n_alleles_total
+  CK(cudaMemcpyAsync(e->h_small + 1, off + S, 4, cudaMemcpyDeviceToHost, st));
+  CK(cudaStreamSynchronize(st));
+  GrimbBatch b;
+  memset(&b, 0, sizeof(b));
+  b.n_subjects = S;
+  b.typed_mask = (const uint16_t*)e->gl_mask.p;
+  b.counts = (const uint16_t*)e->gl_counts.p;
+  b.allele_off = off;
+  b.alleles = (const uint16_t*)e->gl_alleles.p;
+  b.n_alleles_total = (int64_t)(uint32_t)e->h_small[1];
+  b.prior_index = prior_index;
+  b.priors = priors;
+  b.n_priors = n_priors;
+  b.phase_mask = phase_mask;
+  *out = b;
+  return GRIMB_OK;
+}
+
 // What the row decoder needs of the configuration, by value.
 struct RowsCfg {
-  int32_t L, out_u, out_p, n_results, n_pop_results;
+  int32_t L, out_u, out_p, n_results, n_pop_results, hap_pop_pair;
 };
 
 // Per-subject view of a result record (GrimbCompact + its words or its GrimbSubjectResult), the one place
@@ -3929,6 +4107,14 @@ __global__ void __launch_bounds__(256) k_rows_fill(GrimbResults R, RowsCfg c, in
       }
       pmp[q] = h.prob;
     }
+    if (c.hap_pop_pair) {   // the companion pop row of PMUG row q, after the UMUG and PMUG pop rows
+      const GrimbPopRow* cp = R.pop_rows + g.pop_off + g.n_umug_pops + g.n_pmug_pops;
+      for (uint32_t q = 0; q < r.n[1]; ++q) {
+        const GrimbPopRow p = cp[q];
+        O.pmug_pairs[(o[1] + q) * 2] = p.pop_a;
+        O.pmug_pairs[(o[1] + q) * 2 + 1] = p.pop_b;
+      }
+    }
     for (int k = 2; k < 4; ++k) {
       const uint64_t base = g.pop_off + (k == 3 ? g.n_umug_pops : 0u);
       for (uint32_t q = 0; q < r.n[k]; ++q) {
@@ -3991,6 +4177,7 @@ __global__ void __launch_bounds__(256) k_rows_fill(GrimbResults R, RowsCfg c, in
 extern "C" int grimb_results_rows(GrimbEngine* e, const GrimbConfig* cfg, const GrimbBatch* batch, const GrimbResults* res,
                                   const GrimbRows* rows, void* cuda_stream) {
   if (!e || !cfg || !batch || !res || !rows || !rows->totals) return fail(GRIMB_E_ARG, "null argument");
+  if (cfg->hap_pop_pair && !rows->pmug_pairs) return fail(GRIMB_E_ARG, "GrimbRows.pmug_pairs is required under hap_pop_pair");
   const int64_t S = batch->n_subjects;
   if (S < 0 || S > 0x7FFFFFF0ll) return fail(GRIMB_E_ARG, "bad n_subjects");
   for (int k = 0; k < 4; ++k)
@@ -4010,6 +4197,7 @@ extern "C" int grimb_results_rows(GrimbEngine* e, const GrimbConfig* cfg, const 
   c.out_p = cfg->output_pmug ? 1 : 0;
   c.n_results = cfg->n_results;
   c.n_pop_results = cfg->n_pop_results;
+  c.hap_pop_pair = cfg->hap_pop_pair ? 1 : 0;
   e->ev_rows_valid = 0;
   for (int k = 0; k < 4; ++k) CK(cudaMemsetAsync(rows->off[k] + S, 0, 8, st));
   CK(e->geno_small.reserve(64 + sizeof(GenoParams)));

@@ -164,7 +164,7 @@ class Rows(C.Structure):
         ("status", C.c_void_p), ("plan_umug", C.c_void_p), ("plan_pmug", C.c_void_p), ("flags", C.c_void_p),
         ("tot_umug", C.c_void_p), ("tot_pmug", C.c_void_p),
         ("off", C.c_void_p * 4), ("rows", C.c_void_p * 4), ("prob", C.c_void_p * 4), ("capacity", C.c_int64 * 4),
-        ("totals", C.c_void_p),
+        ("totals", C.c_void_p), ("pmug_pairs", C.c_void_p),
     ]
 
 
@@ -240,6 +240,9 @@ def load(kw=1):
                                               C.POINTER(FileStats)]
     lib.grimb_batch_from_genotypes.argtypes = [C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p, C.c_int32,
                                                C.c_void_p, C.POINTER(Batch), C.c_void_p]
+    lib.grimb_batch_from_genotype_lists.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64, C.c_int64, C.c_void_p,
+                                                    C.c_void_p, C.c_int32, C.c_void_p, C.c_void_p, C.POINTER(Batch),
+                                                    C.c_void_p]
     lib.grimb_results_rows.argtypes = [C.c_void_p, C.POINTER(Config), C.POINTER(Batch), C.POINTER(Results),
                                        C.POINTER(Rows), C.c_void_p]
     if lib.grimb_abi_version() != 5:
@@ -270,4 +273,5 @@ EXPORTED = [
     "grimb_text_create", "grimb_text_free", "grimb_text_tokenise", "grimb_text_format", "grimb_impute_text",
     "grimb_impute_file", "grimb_file_count_lines", "grimb_file_write_at", "grimb_file_board_bytes",
     "grimb_impute_file_sharded", "grimb_batch_from_genotypes", "grimb_results_rows",
+    "grimb_batch_from_genotype_lists",
 ]

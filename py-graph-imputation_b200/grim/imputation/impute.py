@@ -302,11 +302,8 @@ class Imputation(object):
         b.alleles, b.n_alleles_total = alle.ctypes.data, int(off[S])
         b.prior_index, b.priors, b.n_priors = pri.ctypes.data, priors.ctypes.data, priors.shape[0]
         b.phase_mask = pmask.ctypes.data if self.phase_masks is not None else None
-        hap_cap = max(1024, S * 2 * min(self.cfg.n_results, 16))
-        pop_cap = max(1024, S * 2 * min(self.cfg.n_pop_results, 4))
-        if self._em_mr:
-            pop_cap += S * min(self.cfg.n_results, 16)
-        res = _lib.ResultArrays(S, self.netGraph.kw, words=max(1024, S * 8), general=max(1024, S), hap=hap_cap, pop=pop_cap)
+        words, general, hap, pop = self._result_caps(S, self._em_mr)
+        res = _lib.ResultArrays(S, self.netGraph.kw, words=words, general=general, hap=hap, pop=pop)
         while True:
             t0 = time.perf_counter()
             rc = self._backend(self.cfg, b, res.struct, workspace)
@@ -318,6 +315,16 @@ class Imputation(object):
                 _lib.check(rc, "grimb_impute_host", self.netGraph.lib)
             break
         return res
+
+    def _result_caps(self, S, em_mr):
+        """First-attempt capacities of the result arrays of a batch of S subjects that may be ambiguous (words,
+        general records, hap rows, pop rows): one general record per subject and the configured number of rows, so
+        that such a batch rarely meets GRIMB_E_CAPACITY, which the library reports only after the kernels ran."""
+        hap = max(1024, S * 2 * min(self.cfg.n_results, 16))
+        pop = max(1024, S * 2 * min(self.cfg.n_pop_results, 4))
+        if em_mr:
+            pop += S * min(self.cfg.n_results, 16)   # the hap_pop_pair companion rows
+        return [max(1024, S * 8), max(1024, S), hap, pop]
 
     # ------------------------------------------------------------------ formatting
     def _allele_name(self, l, i, unknown):
@@ -504,10 +511,7 @@ class Imputation(object):
             mask, counts, flat, unknown = payload
             pm = 0xFFFF
             if binary is not None:
-                pm = 0
-                for m, e in enumerate(binary):
-                    if e == 1 and m < 16:
-                        pm |= 1 << m
+                pm = _phase_mask(binary)
             had_masks = self.phase_masks
             if binary is not None and had_masks is None:
                 self.phase_masks = {}      # makes _run_batch hand the mask array to the kernels
@@ -563,10 +567,7 @@ class Imputation(object):
                 if bits is None:
                     hclass = H_FAULT                   # KeyError f_bin[subject_id] -> raw line in .problem
                 else:
-                    pm = 0
-                    for m, e in enumerate(bits):
-                        if e == 1 and m < 16:
-                            pm |= 1 << m
+                    pm = _phase_mask(bits)
             if len(fields) < 2 or len(fields) == 3 or hclass == H_FAULT:
                 hclass = H_FAULT                       # IndexError in the reference's line parser
             else:
@@ -663,15 +664,65 @@ class Imputation(object):
                     k += 2
         return ids, unknown, text_path
 
+    def encode_genotype_lists(self, gl_strings):
+        """GL strings -> (counts uint16 [S][L][2], alleles uint16 [N], unknown-name maps, text-path line indices) for
+        impute_genotype_lists.  counts[s, l, x] = the number of ids listed on side x of locus l (0/0: untyped);
+        alleles = the ids concatenated subject-major, locus ascending, side 0 then side 1, each list in the order it
+        was written with repeats dropped; unknown[s] as in encode_genotypes.  A line the tokeniser classes as a
+        problem or a fault, or one naming a locus foreign to the table, gets zero counts (it comes back SKIPPED) and
+        its index is listed in the fourth value: such lines belong on the text path (impute_text)."""
+        S, L = len(gl_strings), self.L
+        counts = np.zeros((S, L, 2), np.uint16)
+        unknown = [None] * S
+        text_path = []
+        flat = []
+        for s, gl in enumerate(gl_strings):
+            hclass, payload = self._encode_gl(gl) if gl else (H_PROBLEM, None)
+            if hclass != H_OK or payload == "foreign":
+                text_path.append(s)
+                continue
+            _mask, counts[s], ids, unknown[s] = payload
+            flat.extend(ids)
+        return counts, np.array(flat, np.uint16), unknown, text_path
+
+    def phase_masks_for(self, subject_ids):
+        """Phase masks of the configured bin_imputation_in_file for these subject ids, built as impute_lines builds
+        them: -> (uint16 [S] for the phase_mask argument of impute_genotype_lists, indices of the ids the file has
+        no entry for).  Those subjects get 0xFFFF here; the text path faults their lines (raw line in .problem)."""
+        if self.phase_masks is None:
+            raise ValueError("no bin_imputation_in_file is configured")
+        masks = np.full(len(subject_ids), 0xFFFF, np.uint16)
+        missing = []
+        for s, sid in enumerate(subject_ids):
+            bits = self.phase_masks.get(sid)
+            if bits is None:
+                missing.append(s)
+            else:
+                masks[s] = _phase_mask(bits)
+        return masks, missing
+
     def _check_genotype_modes(self, em_mr, em):
         if em_mr or self.cfg.hap_pop_pair:
-            raise NotImplementedError("impute_genotypes: the hap_pop_pair / em_mr output mode stays on the text path")
+            raise NotImplementedError("impute_genotypes: the hap_pop_pair / em_mr output mode takes impute_genotype_lists")
         if em or self.cfg.em:
-            raise NotImplementedError("impute_genotypes: the em mode stays on the text path")
+            raise NotImplementedError("impute_genotypes: the em mode takes impute_genotype_lists")
         if self.cfg.encounter_order:
             raise NotImplementedError("impute_genotypes: encounter_order (the impute_one seam) stays on impute_one")
         if self.phase_masks is not None:
-            raise NotImplementedError("impute_genotypes: bin_imputation_in_file phase masks stay on the text path")
+            raise NotImplementedError("impute_genotypes: bin_imputation_in_file phase masks take impute_genotype_lists")
+
+    @staticmethod
+    def _device_int16(x, dev, what):
+        """numpy array or CUDA tensor on `dev` -> contiguous CUDA int16 tensor with the same 16-bit patterns."""
+        import torch
+        if isinstance(x, torch.Tensor):
+            if not x.is_cuda or x.device != dev:
+                raise ValueError("%s must be a numpy array or a CUDA tensor on the table's device (%s)" % (what, dev))
+            t = x
+        else:
+            t = torch.from_numpy(np.ascontiguousarray(x))
+        t = t.view(torch.int16) if t.dtype in (torch.uint16, torch.int16) else t.to(torch.int32).to(torch.int16)
+        return t.to(dev).contiguous()
 
     def impute_genotypes(self, ids, prior_index=None, em_mr=False, em=False):
         """Imputes a batch of typed genotypes on the device: ids [S][L][2] allele ids as encode_genotypes returns
@@ -679,20 +730,99 @@ class Imputation(object):
         [S] optional (Imputation.prior_index).  The batch is encoded, imputed and decoded on the GPU
         (grimb_batch_from_genotypes, the imputation kernels, grimb_results_rows).  A CUDA torch tensor on the
         table's device stays there and the results are CUDA tensors; a numpy array gives numpy results.
-        -> GenotypeResults.  Subjects that overflow a workspace tier are re-issued on the next one."""
+        -> GenotypeResults.  Subjects that overflow a workspace tier are re-issued on the next one.  Ambiguous
+        genotypes, phase masks and the EM modes take impute_genotype_lists."""
         import torch
         self._check_genotype_modes(em_mr, em)
         g = self.netGraph
         dev = torch.device("cuda", g.device)
         as_numpy = not isinstance(ids, torch.Tensor)
-        t = torch.from_numpy(np.ascontiguousarray(ids)) if as_numpy else ids
+        t = self._device_int16(ids, dev, "ids")
         if t.dim() != 3 or t.shape[1] != self.L or t.shape[2] != 2:
             raise ValueError("ids must be [S][%d][2]" % self.L)
-        if not as_numpy and (not t.is_cuda or t.device != dev):
-            raise ValueError("ids must be a numpy array or a CUDA tensor on the table's device (%s)" % dev)
-        t = t.view(torch.int16) if t.dtype in (torch.uint16, torch.int16) else t.to(torch.int32).to(torch.int16)
-        t = t.to(dev).contiguous()
-        S = int(t.shape[0])
+        ta = self.type_allowed.ctypes.data if self.type_allowed is not None else None
+        self.cfg.hap_pop_pair = self.cfg.em = 0
+
+        def encoder(todo):
+            sub = t if todo is None else t.index_select(0, todo).contiguous()
+            n = int(sub.shape[0])
+
+            def encode(eng, pri, priors, b, sp):
+                _lib.check(g.lib.grimb_batch_from_genotypes(eng, sub.data_ptr(), n, pri, priors.data_ptr(), priors.shape[0],
+                                                            ta, C.byref(b), sp), "grimb_batch_from_genotypes", g.lib)
+            return n, encode
+        # typed subjects are mostly SIMPLE / TYPED records: few general records and hap rows
+        caps = lambda n: [n * 2 + 1024, n // 8 + 1024, n // 4 + 1024, n // 4 + 1024]
+        return self._impute_device(encoder, int(t.shape[0]), prior_index, dev, as_numpy, caps)
+
+    def impute_genotype_lists(self, counts, alleles, prior_index=None, phase_mask=None, em_mr=False, em=False):
+        """Imputes a batch of genotypes with allele ambiguity on the device: counts [S][L][2] and alleles [N] as
+        encode_genotype_lists returns them (a side's list repeating an id is fine: the repeat is dropped),
+        prior_index [S] optional (Imputation.prior_index), phase_mask [S] optional (uint16, bit m = the m-th typed
+        locus may switch sides; Imputation.phase_masks_for builds it from the configured bin_imputation_in_file,
+        and then it is required).  em_mr: the hap_pop_pair output mode (GenotypeResults.pmug_pairs gets each PMUG
+        row's two populations); em: no Plan C for the haplotype output; both for this call only.  The batch is
+        encoded (grimb_batch_from_genotype_lists), imputed and decoded on the GPU.  CUDA tensors on the table's
+        device stay there and the results are CUDA tensors; numpy counts give numpy results.  -> GenotypeResults.
+        The counts must list N ids in all (ValueError / RuntimeError otherwise).  Subjects that overflow a
+        workspace tier are re-issued on the next one."""
+        import torch
+        if self.cfg.encounter_order:
+            raise NotImplementedError("impute_genotype_lists: encounter_order (the impute_one seam) stays on impute_one")
+        if self.phase_masks is not None and phase_mask is None:
+            raise ValueError("bin_imputation_in_file is configured: pass phase_mask (Imputation.phase_masks_for)")
+        g = self.netGraph
+        dev = torch.device("cuda", g.device)
+        as_numpy = not isinstance(counts, torch.Tensor)
+        c = self._device_int16(counts, dev, "counts")
+        a = self._device_int16(alleles, dev, "alleles")
+        if c.dim() != 3 or c.shape[1] != self.L or c.shape[2] != 2:
+            raise ValueError("counts must be [S][%d][2]" % self.L)
+        if a.dim() != 1:
+            raise ValueError("alleles must be one-dimensional")
+        S = int(c.shape[0])
+        pm = None
+        if phase_mask is not None:
+            pm = self._device_int16(phase_mask, dev, "phase_mask")
+            if tuple(pm.shape) != (S,):
+                raise ValueError("phase_mask must be [S]")
+        ta = self.type_allowed.ctypes.data if self.type_allowed is not None else None
+
+        def encoder(todo):
+            sc, sa, spm = c, a, pm
+            if todo is not None:
+                # the re-issued subjects' lists, gathered from their input offsets
+                n_in = (c.to(torch.int32) & 0xFFFF).sum((1, 2)).to(torch.int64)
+                in_off = torch.cumsum(n_in, 0) - n_in
+                cnt = n_in.index_select(0, todo)
+                total = int(cnt.sum())
+                owner = torch.repeat_interleave(torch.arange(todo.numel(), device=dev), cnt, output_size=total)
+                first = torch.cumsum(cnt, 0) - cnt
+                src = in_off.index_select(0, todo)[owner] + torch.arange(total, device=dev) - first[owner]
+                sc, sa = c.index_select(0, todo).contiguous(), a.index_select(0, src).contiguous()
+                spm = pm.index_select(0, todo).contiguous() if pm is not None else None
+            n = int(sc.shape[0])
+
+            def encode(eng, pri, priors, b, sp):
+                _lib.check(g.lib.grimb_batch_from_genotype_lists(
+                    eng, sc.data_ptr(), sa.data_ptr(), int(sa.numel()), n, pri, priors.data_ptr(), priors.shape[0],
+                    spm.data_ptr() if spm is not None else None, ta, C.byref(b), sp), "grimb_batch_from_genotype_lists", g.lib)
+            return n, encode
+        saved = (self.cfg.hap_pop_pair, self.cfg.em)
+        self.cfg.hap_pop_pair, self.cfg.em = (1 if em_mr else 0), (1 if em else 0)
+        try:
+            return self._impute_device(encoder, S, prior_index, dev, as_numpy,
+                                       lambda n: self._result_caps(n, bool(em_mr)))
+        finally:
+            self.cfg.hap_pop_pair, self.cfg.em = saved
+
+    def _impute_device(self, encoder, S, prior_index, dev, as_numpy, result_caps):
+        """The tier loop of impute_genotypes / impute_genotype_lists.  encoder(todo) -> (n, encode) for the subjects
+        `todo` (CUDA int64 indices; None = the whole batch), where encode(engine, prior_index pointer, priors, batch,
+        stream) builds their batch on the device; result_caps(n) -> the first-attempt capacities of their result
+        arrays (words, general records, hap rows, pop rows)."""
+        import torch
+        g = self.netGraph
         pidx = self._prior_for(None, None)   # the matrix of a line without race fields (and priors never empty)
         if prior_index is None:
             pri = None if pidx == 0 else torch.full((S,), pidx, dtype=torch.int32, device=dev)
@@ -703,14 +833,14 @@ class Imputation(object):
             pri = pri.to(device=dev, dtype=torch.int32).contiguous()
         priors = torch.from_numpy(np.ascontiguousarray(np.stack(self._priors))).to(dev)
         stream = torch.cuda.current_stream(dev)
-        self.cfg.hap_pop_pair = self.cfg.em = 0
         out = None
         todo = None   # indices of the subjects re-issued on this tier (None: the whole batch)
-        retries = 0
+        retries = reruns = 0
         for tier in self.workspaces:
-            sub_ids = t if todo is None else t.index_select(0, todo).contiguous()
+            n, encode = encoder(todo)
             sub_pri = pri if (pri is None or todo is None) else pri.index_select(0, todo).contiguous()
-            part = self._genotype_pass(sub_ids, sub_pri, priors, tier, stream)
+            part = self._genotype_pass(encode, n, sub_pri, priors, tier, stream, result_caps(n))
+            reruns += part.pop("capacity_reruns")
             out = part if todo is None else _splice_rows(out, part, todo)
             again = (part["status"] == _lib.ST_WORKSPACE).nonzero().flatten()
             if again.numel() == 0:
@@ -729,24 +859,23 @@ class Imputation(object):
                 raise NotImplementedError(
                     "subject %d leaves Plan A without a result under a Plan_A_Matrix: the reference's Plan B is not "
                     "well defined there; set \"planb\": false to write such subjects to the .miss file" % s)
+        out["capacity_reruns"] = reruns
         return GenotypeResults(out, g.alleles, self.populations, retries, as_numpy)
 
-    def _genotype_pass(self, ids, pri, priors, tier, stream):
-        """One tier: encode, impute and decode `ids` (CUDA int16 [S][L][2]) -> dict of CUDA tensors."""
+    def _genotype_pass(self, encode, S, pri, priors, tier, stream, caps):
+        """One tier: encode (see _impute_device), impute and decode S subjects -> dict of CUDA tensors, and the
+        number of times grimb_impute_device ran again on larger result arrays ("capacity_reruns")."""
         import torch
         g, lib = self.netGraph, self.netGraph.lib
-        dev = ids.device
+        dev = priors.device
         eng = g.engine(tier)
-        S, L = int(ids.shape[0]), self.L
+        L = self.L
         sp = C.c_void_p(stream.cuda_stream)
         b = _lib.Batch()
-        ta = self.type_allowed.ctypes.data if self.type_allowed is not None else None
-        _lib.check(lib.grimb_batch_from_genotypes(eng, ids.data_ptr(), S, pri.data_ptr() if pri is not None else None,
-                                                  priors.data_ptr(), priors.shape[0], ta, C.byref(b), sp),
-                   "grimb_batch_from_genotypes", lib)
+        encode(eng, pri.data_ptr() if pri is not None else None, priors, b, sp)
         hap_sz = 24 if g.kw == 1 else 40
-        caps = [S * 2 + 1024, S // 8 + 1024, S // 4 + 1024, S // 4 + 1024]
         totals = np.zeros(9, np.int64)
+        reruns = 0
         while True:
             compact = torch.empty(max(1, S) * 16, dtype=torch.uint8, device=dev)
             bufs = [torch.empty(c * sz, dtype=torch.uint8, device=dev) for c, sz in zip(caps, (8, 48, hap_sz, 16))]
@@ -759,20 +888,25 @@ class Imputation(object):
             rc = lib.grimb_impute_device(eng, C.byref(self.cfg), C.byref(b), C.byref(r), sp)
             if rc == _lib.E_CAPACITY:
                 caps = [max(c, int(x)) for c, x in zip(caps, totals[:4])]
+                reruns += 1
                 continue
             _lib.check(rc, "grimb_impute_device", lib)
             break
         out = {"status": torch.empty(S, dtype=torch.uint8, device=dev), "plan_umug": torch.empty(S, dtype=torch.uint8, device=dev),
                "plan_pmug": torch.empty(S, dtype=torch.uint8, device=dev), "flags": torch.empty(S, dtype=torch.uint8, device=dev),
                "tot_umug": torch.empty(S, dtype=torch.int32, device=dev), "tot_pmug": torch.empty(S, dtype=torch.int32, device=dev),
-               "pair_evals": int(totals[4])}
+               "pair_evals": int(totals[4]), "capacity_reruns": reruns}
         for k in _lib.ROW_KINDS:
             out[k + "_off"] = torch.empty(S + 1, dtype=torch.int64, device=dev)
         width = (2 * L, 2 * L, 2, 2)
         rcap = list(getattr(self, "_row_caps", (S + 1024, 2 * S + 1024, S + 1024, S + 1024)))
         rtot = np.zeros(4, np.int64)
+        pairs = bool(self.cfg.hap_pop_pair)
         while True:
             rows = _lib.Rows()
+            if pairs:
+                out["pmug_pairs"] = torch.empty((rcap[1], 2), dtype=torch.int16, device=dev)
+                rows.pmug_pairs = out["pmug_pairs"].data_ptr()
             for f in ("status", "plan_umug", "plan_pmug", "flags", "tot_umug", "tot_pmug"):
                 setattr(rows, f, out[f].data_ptr())
             for i, k in enumerate(_lib.ROW_KINDS):
@@ -791,6 +925,8 @@ class Imputation(object):
         for i, k in enumerate(_lib.ROW_KINDS):
             out[k] = out[k][:int(rtot[i])].reshape((int(rtot[i]),) + shapes[i])
             out[k + "_prob"] = out[k + "_prob"][:int(rtot[i])]
+        if pairs:
+            out["pmug_pairs"] = out["pmug_pairs"][:int(rtot[1])]
         return out
 
     # ------------------------------------------------------------------ EM helpers (host only)
@@ -1057,6 +1193,15 @@ class Imputation(object):
                 f.writelines(files[k])
 
 
+def _phase_mask(bits):
+    """A bin_imputation_in_file entry (one 0/1 per typed locus) -> the GrimbBatch.phase_mask word."""
+    pm = 0
+    for m, e in enumerate(bits):
+        if e == 1 and m < 16:
+            pm |= 1 << m
+    return pm
+
+
 _SUBJECT_FIELDS = ("status", "plan_umug", "plan_pmug", "flags", "tot_umug", "tot_pmug")
 
 
@@ -1085,14 +1230,20 @@ def _splice_rows(base, part, idx):
         prob = torch.empty(total, dtype=torch.float64, device=dev)
         src = po[p[mine]] + within[mine]
         rows[mine], prob[mine] = part[k][src], part[k + "_prob"][src]
+        psrc = src
         src = bo[owner[~mine]] + within[~mine]
         rows[~mine], prob[~mine] = base[k][src], base[k + "_prob"][src]
         out[k], out[k + "_prob"], out[k + "_off"] = rows, prob, off
+        if k == "pmug" and "pmug_pairs" in base:
+            pairs = torch.empty((total, 2), dtype=base["pmug_pairs"].dtype, device=dev)
+            pairs[mine], pairs[~mine] = part["pmug_pairs"][psrc], base["pmug_pairs"][src]
+            out["pmug_pairs"] = pairs
     return out
 
 
 class GenotypeResults(object):
-    """Result of Imputation.impute_genotypes: ragged rows in input order (include/grimb200.h, GrimbRows).
+    """Result of Imputation.impute_genotypes / impute_genotype_lists: ragged rows in input order (include/grimb200.h,
+    GrimbRows).
 
     Per subject [S]: status (GRIMB_ST_*), plan_umug, plan_pmug (GRIMB_PLAN_*), tot_umug, tot_pmug (the counts the
     reference prints), flags (bit 0 has results, bit 1 written to .miss, bit 2 written to .problem).
@@ -1100,13 +1251,17 @@ class GenotypeResults(object):
     k_off[s]:k_off[s+1], in rank order), k (uint16 rows: umug [n][L][2] (min id, max id) allele pairs, pmug [n][2][L]
     haplotype 1 / haplotype 2 (0 = no allele), pop kinds [n][2] population indices, 0xFFFF = all_pops) and k_prob
     [n] (float64).  alleles[l][id - 1] names table allele `id` of locus l; populations[p] names population p.
-    pair_evals: pair evaluations of the batch; workspace_retries: subjects re-issued on a bigger workspace tier.
+    pmug_pairs [n_pmug][2]: under em_mr (impute_genotype_lists), the populations of haplotype 1 and haplotype 2 of
+    each PMUG row (the hap;pop pairs of the reference's hap_pop_pair output); None otherwise.
+    pair_evals: pair evaluations of the batch; workspace_retries: subjects re-issued on a bigger workspace tier;
+    capacity_reruns: times the imputation ran again because its result arrays were too small (0 normally).
     Arrays are CUDA tensors when the input was one, numpy arrays otherwise."""
 
     def __init__(self, d, alleles, populations, workspace_retries, as_numpy):
         import torch
         self.alleles, self.populations = alleles, populations
         self.pair_evals, self.workspace_retries = d["pair_evals"], workspace_retries
+        self.capacity_reruns = d["capacity_reruns"]
         for f in _SUBJECT_FIELDS:
             v = d[f]   # uint8, or int32 storage of the uint32 totals
             if as_numpy:
@@ -1119,6 +1274,8 @@ class GenotypeResults(object):
             setattr(self, k, rows.cpu().numpy().view(np.uint16) if as_numpy else rows.view(torch.uint16))
             setattr(self, k + "_prob", d[k + "_prob"].cpu().numpy() if as_numpy else d[k + "_prob"])
             setattr(self, k + "_off", d[k + "_off"].cpu().numpy() if as_numpy else d[k + "_off"])
+        pp = d.get("pmug_pairs")
+        self.pmug_pairs = None if pp is None else (pp.cpu().numpy().view(np.uint16) if as_numpy else pp.view(torch.uint16))
 
     def __len__(self):
         return int(self.status.shape[0])
